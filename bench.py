@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: TPC-H Q1/Q6/Q3 pipelines on TPC-H-shaped synthetic data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--sf SF] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--sf SF] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): lineitem tuples/s over Q1+Q6+Q3 at SF100 (+ fraction of the HBM roofline).
 A step = one pass of the three queries over the resident tables (3 scans of lineitem plus the
@@ -31,6 +31,32 @@ QUERIES = ("q1", "q6", "q3")
 def load_plan(name):
     with open(os.path.join(ROOT, "tests/golden/plans", name + ".json")) as f:
         return json.load(f)
+
+
+def dump_outputs(out_dir, results, max_bytes=64 << 20):
+    """Writes the result columns a caller of rq_plan_execute received, one `<query>.<column>.npy` per
+    column, so that two builds can be compared output for output on the same seeded inputs. Integer
+    columns (DECIMAL as scaled integers) become float64, strings a (rows, width) float32 array of their
+    bytes. A result larger than its share of `max_bytes` is reduced to a fixed, seeded sample of rows,
+    the same rows in every column, whose indices go to `<query>.rows.npy`."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for q, res in results.items():
+        names = res.names or [f"col{i}" for i in range(len(res.columns))]
+        row_bytes = 8 + sum(8 if c.dtype.kind != "S" else 4 * c.dtype.itemsize for c in res.columns)
+        keep = (max_bytes // len(results)) // row_bytes
+        rows = None
+        if res.n_rows > keep:
+            rows = np.sort(np.random.default_rng(0).choice(res.n_rows, size=keep, replace=False))
+            np.save(os.path.join(out_dir, f"{q}.rows.npy"), rows.astype(np.float64))
+        for i, (name, col) in enumerate(zip(names, res.columns)):
+            if rows is not None:
+                col = col[rows]
+            if col.dtype.kind == "S":
+                arr = col.view(np.uint8).reshape(len(col), col.dtype.itemsize).astype(np.float32)
+            else:
+                arr = col.astype(np.float64)
+            np.save(os.path.join(out_dir, f"{q}.{i:02d}_{name}.npy"), arr)
 
 
 def measured_peak():
@@ -208,7 +234,7 @@ def main_micro(a):
 
         times, res, tm = [], None, None
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        reps = 1 + max(a.warmup, 2) + max(1, min(a.steps, 5))
+        reps = 1 + max(a.warmup, 2) + a.steps
         for i in range(reps):
             barrier()
             t0 = time.perf_counter()
@@ -221,6 +247,8 @@ def main_micro(a):
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
             times.append(t.tolist())
         timed = times[1 + max(a.warmup, 2):]
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, {f"micro_n{n}_g{g}": res}, (64 << 20) // len(cases))
         # ---- independent evaluation ------------------------------------------------------------
         s = torch.zeros(g, dtype=torch.int64, device=dev).index_add_(0, foo_c, foo_a * foo_a)
         k = torch.zeros(g, dtype=torch.int64, device=dev).index_add_(0, foo_c, torch.ones_like(foo_a))
@@ -291,7 +319,7 @@ def main_joins(a):
         plan = Plan(d)
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         times, walls = [], []
-        reps = 1 + max(a.warmup, 3) + max(3, min(a.steps, 10))
+        reps = 1 + max(a.warmup, 3) + a.steps
         for i in range(reps):
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -301,6 +329,8 @@ def main_joins(a):
             torch.cuda.synchronize()
             times.append(ev0.elapsed_time(ev1)); walls.append(1e3 * (time.perf_counter() - t0))
         timed = times[1 + max(a.warmup, 3):]
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {q: res}, (64 << 20) // 3)
         got = serialize_columns(res.columns, res.sql_types, res.sql_widths)
         want = serialize_columns(*run_plan(d, tabs))
         order = d.get("order", [])
@@ -327,7 +357,7 @@ def main_joins(a):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (every timed loop runs exactly this many)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--sf", type=float, default=float(os.environ.get("RESQL_BENCH_SF", "100")))
     ap.add_argument("--impl", default="ours")
@@ -338,7 +368,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--workload", default="tpch", choices=["tpch", "micro", "joins"])
     ap.add_argument("--micro-cases", default="", help="N:G,N:G,... (default: 1e8 x {4,1e6,1e8}; with >= 4 GPUs also 1e9)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the results of the last step as DIR/<query>.<column>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.workload == "micro":
         return main_micro(a)
     if a.workload == "joins":
@@ -468,6 +502,8 @@ def main():
         barrier()
     dt = max_over_ranks(ev0.elapsed_time(ev1) / 1e3)      # device time on the engine stream
     last = r
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {q: last[q][0] for q in QUERIES})
     clocks = clk.summary()
     value = 3.0 * n_total * a.steps / dt
 
@@ -608,7 +644,7 @@ def main():
 
         for _ in range(2):
             step_e2e()
-        e_steps = max(2, min(a.steps, 5))
+        e_steps = a.steps
         barrier()
         ev0.record(stream)
         for _ in range(e_steps):
