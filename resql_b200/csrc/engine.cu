@@ -143,7 +143,7 @@ struct Engine {
     int64_t* g_keys = nullptr;
     int64_t* g_acc = nullptr;
     uint8_t* g_kinds = nullptr;
-    int32_t* flags = nullptr;   // [0]=overflow [1]=ht_full [2]=err
+    int32_t* flags = nullptr;   // FlagBlock (rq_internal.h), 64 bytes
     int32_t* h_flags = nullptr; // pinned
     unsigned char* pinned = nullptr;   // pinned scratch: host reads (4 KB) + ring of small uploads
     Dist dist;

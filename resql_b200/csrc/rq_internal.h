@@ -1,6 +1,7 @@
 // Internal (host+device) definitions of the resql_b200 engine. Not part of the ABI.
 #pragma once
 #include <stdint.h>
+#include <stddef.h>
 
 namespace rq {
 
@@ -35,6 +36,42 @@ enum AggMode : uint8_t { AM_FULL = 0, AM_P1 = 1, AM_P2 = 2, AM_W64 = 3 };
 enum AggForm : uint32_t { AF_NONE = 0, AF_P1 = 1, AF_P2 = 2, AF_W64 = 3, AF_FULL = 4, AF_MIN = 5, AF_MAX = 6 };
 
 enum SinkImpl { IMPL_LOWAGG = 1, IMPL_HASHAGG = 2, IMPL_BUILD = 3, IMPL_EMIT = 4, IMPL_REGAGG = 5 };
+
+// ---- status words of a pipeline launch ----------------------------------------------------------
+// One block in device memory (Engine::flags, 64 bytes) that kernels raise and count into, and its
+// pinned host copy the host reads back after a launch.
+struct FlagBlock {
+    int32_t  overflow;      // a warp met more groups than its aggregation path tracks
+    int32_t  ht_full;       // hash table full, or past the load a launch may add
+    int32_t  err;           // 1: division by zero, 2: probe in a kernel variant without probe code
+    int32_t  dup_key;       // direct-address build: duplicate key, or a key outside the domain
+    uint64_t dup_matches;   // multi-match probe: tuples with more than one match
+    uint64_t entries;       // hash / direct-address table entries the launch added
+    uint64_t extra;         // a device word copied behind the flags so one read brings both
+    uint64_t reserved;
+    uint64_t popcount;      // shared build: set bits of the all-reduced bitmap
+};
+static_assert(offsetof(FlagBlock, overflow) == 0, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, ht_full) == 4, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, err) == 8, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, dup_key) == 12, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, dup_matches) == 16, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, entries) == 24, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, extra) == 32, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, reserved) == 40, "FlagBlock layout");
+static_assert(offsetof(FlagBlock, popcount) == 48, "FlagBlock layout");
+static_assert(sizeof(FlagBlock) <= 64, "FlagBlock must fit Engine::flags");
+// The words in front of `extra` are cleared before a launch and, for a shared build, summed over
+// the ranks as four uint64.
+constexpr size_t kFlagsCleared = offsetof(FlagBlock, extra);
+static_assert(kFlagsCleared == 32, "the cleared and summed prefix is four uint64");
+// int32 word indices, for device code that addresses the block through an int32_t*
+constexpr int kFlagWordErr      = offsetof(FlagBlock, err) / 4;
+constexpr int kFlagWordDupKey   = offsetof(FlagBlock, dup_key) / 4;
+constexpr int kFlagWordEntries  = offsetof(FlagBlock, entries) / 4;
+constexpr int kFlagWordPopcount = offsetof(FlagBlock, popcount) / 4;
+// KParams::ht_full points at FlagBlock::ht_full; the direct-address build raises dup_key through it
+constexpr int kDupKeyFromHtFull = (offsetof(FlagBlock, dup_key) - offsetof(FlagBlock, ht_full)) / 4;
 
 // ---- operation codes shared by the host-level program and the device encoding ----------------
 enum DOp : uint8_t {

@@ -1141,8 +1141,8 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     for (int r = 0; r < kR; r++) {
                         if (!((valid >> r) & 1)) continue;
                         const uint64_t idx = (uint64_t)bk[r] - (uint64_t)P.ht.dlo;
-                        if (idx >= P.ht.dsize) { *const_cast<int32_t*>(P.ht_full + 2) = 1; continue; }   // outside the proven domain
-                        if (was[r] & (1u << (idx & 31))) *const_cast<int32_t*>(P.ht_full + 2) = 1;     // duplicate key: the host falls back to the hash form
+                        if (idx >= P.ht.dsize) { *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1; continue; }   // outside the proven domain
+                        if (was[r] & (1u << (idx & 31))) *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1;     // duplicate key: the host falls back to the hash form
                         for (int q = 0; q < P.n_out; q++) P.ht.darr[idx * P.ht.dnv + q] = (uint64_t)ld_row(P, c, P.out[q], r);
                         n_inserted++;
                     }
@@ -1477,15 +1477,15 @@ __global__ void rq_popcount_words(const uint32_t* w, size_t n, unsigned long lon
     c = (unsigned long long)warp_reduce((int64_t)c, 1);
     if ((threadIdx.x & 31) == 0 && c) atomicAdd(out, c);
 }
-// ... must equal the summed entry count (flags words 6-7), else two ranks inserted the same key: raise
-// the duplicate flag (word 3) so that every rank falls back to the hash form
+// ... must equal the summed entry count (FlagBlock::entries), else two ranks inserted the same key:
+// raise FlagBlock::dup_key so that every rank falls back to the hash form
 __global__ void rq_shared_build_check(int32_t* flags) {
     if (threadIdx.x != 0) return;
-    const unsigned long long entries = *reinterpret_cast<unsigned long long*>(flags + 6);
-    const unsigned long long bits = *reinterpret_cast<unsigned long long*>(flags + 12);
-    if (entries != bits) flags[3] = 1;
-    if (flags[2] > 1) flags[2] = 1;         // (error flags were summed over the ranks)
-    if (flags[3] > 1) flags[3] = 1;
+    const unsigned long long entries = *reinterpret_cast<unsigned long long*>(flags + kFlagWordEntries);
+    const unsigned long long bits = *reinterpret_cast<unsigned long long*>(flags + kFlagWordPopcount);
+    if (entries != bits) flags[kFlagWordDupKey] = 1;
+    if (flags[kFlagWordErr] > 1) flags[kFlagWordErr] = 1;         // (error flags were summed over the ranks)
+    if (flags[kFlagWordDupKey] > 1) flags[kFlagWordDupKey] = 1;
 }
 
 // min / max of an integer column (upload-time statistics): out[0] = min, out[1] = max
