@@ -119,6 +119,7 @@ struct Options {
     bool prune_builds = true;             // restrict build sides to the probe key's value range
     bool topk = true;                     // ORDER BY ... LIMIT k through radix select
     bool direct_joins = true;             // direct-address join tables for dense unique integer keys
+    bool group_joins = true;              // GROUP BY on the key of a direct-address join aggregates into its entries
     bool replay = true;                   // predicted host reads (engine_exec.inl "host reads of device values")
     bool graphs = true;                   // replayed plans are captured into CUDA graphs
     bool zone_skip = true;                // selections on sorted columns restrict the scan to a tile range
@@ -245,6 +246,7 @@ extern "C" int rq_set_option(const char* key, double value) {
     else if (k == "prune_builds") o.prune_builds = value != 0;
     else if (k == "topk") o.topk = value != 0;
     else if (k == "direct_joins") o.direct_joins = value != 0;
+    else if (k == "group_joins") o.group_joins = value != 0;
     else if (k == "replay") o.replay = value != 0;
     else if (k == "graphs") o.graphs = value != 0;
     else if (k == "narrow") o.narrow = value != 0;
@@ -766,6 +768,9 @@ struct PipeOut {                    // what a finished pipeline left on the devi
     std::unique_ptr<HashTableDev> ht;  // BUILD output
     std::vector<int> payload_sql_type, payload_sql_width;
     std::vector<uint8_t> pay_word;     // BUILD: payload index (as in the plan) -> entry word, 0xff = not stored
+    bool gj = false;                   // BUILD: direct-address entries carry the accumulators of a groupjoin,
+    std::vector<int> gj_kind;          //        of these aggregate kinds, from entry word gj_word on
+    uint32_t gj_word = 0;
     std::vector<void*> owned;          // device buffers the relation's string addresses point into
     ~PipeOut() { for (void* p : owned) dfree(p); }
     PipeOut() = default;

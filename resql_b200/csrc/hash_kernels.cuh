@@ -232,4 +232,55 @@ __global__ void rq_ht_compact_packed(DHashTable ht, PackedCompact pc, unsigned l
     }
 }
 
+// groupjoin (IMPL_GROUPJOIN): the touched entries of a direct-address table -> dense int64 columns.
+// word[c] < 0 selects the entry's key (dlo + index), otherwise entry word word[c] (a stored payload or
+// an accumulator). A block of kGjThreads threads covers kGjWordsPerThread words per thread of the
+// touched bitmap and takes its output range with ONE atomic: the groups are sparse in the bitmap (Q3
+// at SF100: 1.1 M groups in 18.75 M words), so one atomic per warp would be ~0.5 M atomics on one
+// counter, which serialize.
+constexpr int kGjThreads = 256, kGjWordsPerThread = 8;
+struct GjCompact { int32_t n_out; int16_t word[kMaxOut]; int64_t* out[kMaxOut]; };
+__global__ void __launch_bounds__(kGjThreads) rq_groupjoin_compact(DHashTable ht, const uint32_t* touched, GjCompact gc,
+                                                                   unsigned long long* count, unsigned long long out_cap) {
+    __shared__ int warp_off[kGjThreads / 32];
+    __shared__ unsigned long long block_base;
+    const uint64_t words = (ht.dsize + 31) / 32;
+    const uint64_t w0 = (uint64_t)blockIdx.x * kGjThreads * kGjWordsPerThread + threadIdx.x;
+    uint32_t w[kGjWordsPerThread];
+    int n = 0;
+#pragma unroll
+    for (int j = 0; j < kGjWordsPerThread; j++) {
+        const uint64_t i = w0 + (uint64_t)j * kGjThreads;
+        w[j] = i < words ? touched[i] : 0u;
+        n += __popc(w[j]);
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = n;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) warp_off[warp] = incl;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int t = 0;
+        for (int k = 0; k < kGjThreads / 32; k++) { const int x = warp_off[k]; warp_off[k] = t; t += x; }
+        block_base = t ? atomicAdd(count, (unsigned long long)t) : 0ULL;
+    }
+    __syncthreads();
+    unsigned long long pos = block_base + (unsigned long long)(warp_off[warp] + incl - n);
+#pragma unroll 1
+    for (int j = 0; j < kGjWordsPerThread; j++) {
+        const uint64_t i = w0 + (uint64_t)j * kGjThreads;
+        for (uint32_t b = w[j]; b; b &= b - 1, pos++) {
+            const uint64_t idx = i * 32 + (uint64_t)(__ffs(b) - 1);
+            if (pos >= out_cap) continue;          // (sized from a count the host may only have predicted)
+            const uint64_t* e = ht.darr + idx * ht.dnv;
+            for (int c = 0; c < gc.n_out; c++)
+                gc.out[c][pos] = gc.word[c] < 0 ? ht.dlo + (int64_t)idx : (int64_t)e[gc.word[c]];
+        }
+    }
+}
+
 }  // namespace rq

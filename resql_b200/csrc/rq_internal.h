@@ -35,7 +35,7 @@ enum AggMode : uint8_t { AM_FULL = 0, AM_P1 = 1, AM_P2 = 2, AM_W64 = 3 };
 // what the aggregate loop of the register path does for one aggregate (KParams::agg_desc bits 0-2)
 enum AggForm : uint32_t { AF_NONE = 0, AF_P1 = 1, AF_P2 = 2, AF_W64 = 3, AF_FULL = 4, AF_MIN = 5, AF_MAX = 6 };
 
-enum SinkImpl { IMPL_LOWAGG = 1, IMPL_HASHAGG = 2, IMPL_BUILD = 3, IMPL_EMIT = 4, IMPL_REGAGG = 5 };
+enum SinkImpl { IMPL_LOWAGG = 1, IMPL_HASHAGG = 2, IMPL_BUILD = 3, IMPL_EMIT = 4, IMPL_REGAGG = 5, IMPL_GROUPJOIN = 6 };
 
 // ---- status words of a pipeline launch ----------------------------------------------------------
 // One block in device memory (Engine::flags, 64 bytes) that kernels raise and count into, and its
@@ -176,7 +176,7 @@ struct DHashTable {
     uint32_t  packed;               // hash aggregation: entry = [packed group key + 1][accumulators] (no tag, no key words)
     uint32_t  pad3_;
     uint32_t  direct;
-    uint32_t  dnv;                  // payload words per key
+    uint32_t  dnv;                  // words per key: payloads, then groupjoin accumulators (KParams::gj_acc_word)
     int64_t   dlo;
     uint64_t  dsize;
     uint32_t* dbits;
@@ -261,6 +261,12 @@ struct KParams {
     DHashTable     ht;
     int32_t*       ht_full;              // set when the table is full
     unsigned long long* ht_entries;      // entries added by this launch
+    // groupjoin (IMPL_GROUPJOIN): ht is the probed direct-address table; the aggregates of a tuple go
+    // into words [gj_acc_word, + na) of the entry its key selects. A direct-address build writes the
+    // identities of agg_kind[0 .. na) into those words of every entry it stores.
+    uint32_t*      gj_touched;           // bit per entry: it received a tuple
+    uint32_t       gj_acc_word;
+    int32_t        pad2_;
     // probes
     int32_t        n_probes;
     DProbe         probe[kMaxProbes];

@@ -1144,6 +1144,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         if (idx >= P.ht.dsize) { *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1; continue; }   // outside the proven domain
                         if (was[r] & (1u << (idx & 31))) *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1;     // duplicate key: the host falls back to the hash form
                         for (int q = 0; q < P.n_out; q++) P.ht.darr[idx * P.ht.dnv + q] = (uint64_t)ld_row(P, c, P.out[q], r);
+                        for (int a = 0; a < NA; a++) P.ht.darr[idx * P.ht.dnv + P.gj_acc_word + a] = (uint64_t)agg_identity(P.agg_kind[a]);
                         n_inserted++;
                     }
                 } else if (bnk == 1 && P.ht.key_kind[0] == 0) {
@@ -1243,6 +1244,32 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     if (!ht_find_or_insert(P.ht, k, hh, &slot, &fresh, P.ht_full)) { *P.ht_full = 1; continue; }
                     if (fresh) n_inserted++;
                     uint64_t* acc = ht_entry(P.ht, slot) + 1 + P.ht.nk;
+                    for (int a = 0; a < NA; a++) {
+                        const int kind = P.agg_kind[a];
+                        if (kind == 2) { atomicAdd((unsigned long long*)&acc[a], 1ULL); continue; }
+                        const int64_t v = ld_row(P, c, P.agg_src[a], r);
+                        if (kind == 1) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
+                        else if (kind == 3) atomicMin((long long*)&acc[a], (long long)v);
+                        else atomicMax((long long*)&acc[a], (long long)v);
+                    }
+                }
+            } else if (sink == IMPL_GROUPJOIN) {
+                // GROUP BY on the key of a direct-address join (engine_exec.inl groupjoin_probe): the
+                // probe in front kept only tuples whose key has an entry, and each entry is exactly one
+                // group. A tuple marks its entry touched and adds into the entry's accumulator words
+                // with fire-and-forget atomics; the group's other keys stay in the entry until the
+                // compaction reads them once per group.
+                int64_t gk[kR];
+                fetch_vref(P, c, P.key[0], gk);
+#pragma unroll 1
+                for (int r = 0; r < kR; r++) {
+                    if (!((valid >> r) & 1)) continue;
+                    int64_t k = 0;
+#pragma unroll
+                    for (int q = 0; q < kR; q++) if (q == r) k = gk[q];
+                    const uint64_t idx = (uint64_t)k - (uint64_t)P.ht.dlo;
+                    atomicOr(&P.gj_touched[idx >> 5], 1u << (idx & 31));
+                    uint64_t* acc = P.ht.darr + idx * P.ht.dnv + P.gj_acc_word;
                     for (int a = 0; a < NA; a++) {
                         const int kind = P.agg_kind[a];
                         if (kind == 2) { atomicAdd((unsigned long long*)&acc[a], 1ULL); continue; }
