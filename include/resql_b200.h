@@ -184,8 +184,10 @@ typedef struct {
 #define RQ_SRC_CROSS     3   /* cross product of two earlier materialized pipelines, source_id x
                                 source_id2 (NestedLoopsJoinOp, nestedloopsjoin.h:5-94: both children
                                 are materialized, every pair is produced, an optional condition
-                                follows as RQ_OP_FILTER). COL indices address the columns of
-                                source_id first, then those of source_id2.                       */
+                                follows as RQ_OP_FILTER). The pairs are streamed through the scan
+                                kernel, never materialized; just under 2^40 pairs at most
+                                (RQ_ERR_UNSUPPORTED beyond). COL indices address the columns of source_id first, then
+                                those of source_id2.                                             */
 
 #define RQ_SRC_ONE_ROW   4   /* a single tuple without attributes: leaf projection, "creates a
                                 single-line table from constants" (projection.h:49-58, `select 1+1`) */

@@ -103,6 +103,11 @@ struct rq_table {
     std::vector<DevColumn> cols;
     // logical type info for intermediates (per column)
     std::vector<int> sql_type, sql_width;
+    // nested-loops join source (RQ_SRC_CROSS): the pairs of two relation outputs, streamed by the scan
+    // kernel and never materialized. `cols` aliases the columns of cross[0], then those of cross[1];
+    // n_rows is the pair count; cross[cross_inner] is the relation iterated inside (scan_kernel.cuh)
+    const rq_table* cross[2] = {nullptr, nullptr};
+    int cross_inner = 1;
     ~rq_table() {
         for (auto& c : cols)
             if (c.owned && c.d) dfree(c.d);
@@ -200,6 +205,7 @@ extern "C" int rq_init(int device) {
         CK(cudaFuncSetAttribute(rq_scan_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         CK(cudaFuncSetAttribute(rq_scan_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         CK(cudaFuncSetAttribute(rq_scan_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+        CK(cudaFuncSetAttribute(rq_scan_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         E.init = true;
         return RQ_OK;
     } catch (RqError& e) {
@@ -988,6 +994,9 @@ struct Lowerer {
             for (size_t k = 0; k < staged_of_col.size(); k++)
                 if (src.cols[k].type != RQ_STR && staged_of_col[k] >= 0) src_of[staged_of_col[k]] = (int)k;
             const bool tile_major = src.pax_base != nullptr;
+            const bool cross = src.cross[0] != nullptr;    // no runs: the kernel gathers every column itself
+            const int n_left = cross ? (int)src.cross[0]->cols.size() : 0;
+            P.cross_inner = 0;
             if (tile_major)
                 std::sort(order.begin(), order.end(), [&](int a, int b) { return src.cols[src_of[a]].page_off < src.cols[src_of[b]].page_off; });
             uint32_t off = 0;
@@ -997,7 +1006,9 @@ struct Lowerer {
                 const uint32_t bytes = (uint32_t)kTile * P.col_w[c];
                 P.col_off[c] = off;
                 const int r = P.n_runs - 1;
-                if (tile_major && r >= 0 && P.run_ptr[r] + P.run_bytes[r] == dc.d) {
+                if (cross) {
+                    if ((src_of[c] >= n_left) == (src.cross_inner == 1)) P.cross_inner |= 1u << c;
+                } else if (tile_major && r >= 0 && P.run_ptr[r] + P.run_bytes[r] == dc.d) {
                     P.run_bytes[r] += bytes;              // adjacent in the page: same copy
                 } else {
                     P.run_ptr[P.n_runs] = dc.d;

@@ -281,6 +281,14 @@ struct KParams {
     int64_t        out_cap;
     // runtime error flag (division by zero)
     int32_t*       err;
+    // nested-loops join source (RQ_SRC_CROSS, kernel variant CROSS): pair p of the source is (row
+    // p / n_inner of the outer relation, row p % n_inner of the inner one); every staged column is a
+    // plain int64 array col_ptr[c] of one of the two. (Behind every other field, so that the variants
+    // without it address their parameters exactly as before.)
+    const int64_t* cross_rows[2];        // [outer, inner]: row counts, read on the device ...
+    int64_t        cross_cap[2];         // ... and clamped to the rows each relation has room for
+    uint32_t       cross_inner;          // bit c: staged column c belongs to the inner relation
+    int32_t        pad3_;
 };
 
 }  // namespace rq

@@ -282,9 +282,62 @@ template <> struct ScanCfg<0> { static constexpr int kThreads = 512; };
 template <> struct ScanCfg<1> { static constexpr int kThreads = 512; };
 template <> struct ScanCfg<4> { static constexpr int kThreads = 512; };
 
-template <int GR>
+// Nested-loops join source (CROSS, instantiated with GR = 0 only): the pairs of two relations are
+// never materialized. Tile t holds pairs [256t, 256t + 256); pair p is (outer row p / n_inner, inner
+// row p % n_inner). The host makes the smaller relation the inner one: consecutive pairs sweep the
+// inner relation while the outer row changes once every n_inner pairs, so the columns read again and
+// again are the smaller ones (at most 2^20 rows under the 2^40-pair limit: 8 MB per column, L2
+// resident), and the outer row of a tile is one broadcast load. The warp stages a tile itself with
+// plain loads at the offsets a bulk copy would use; there are no bulk copies and no mbarriers.
+// Row counts are read on the device, clamped to each relation's capacity and to the pair count the
+// host sized the launch for, so a wrong replay prediction cannot gather outside an allocation.
+__device__ __forceinline__ int64_t cross_pairs(const KParams& P, uint64_t& n_inner) {
+    int64_t n[2];
+#pragma unroll
+    for (int k = 0; k < 2; k++) {
+        n[k] = *P.cross_rows[k];
+        n[k] = n[k] < 0 ? 0 : (n[k] > P.cross_cap[k] ? P.cross_cap[k] : n[k]);
+    }
+    n_inner = (uint64_t)n[1];
+    if (n[0] == 0 || n[1] == 0) return 0;
+    return n[1] > P.n_rows / n[0] ? P.n_rows : n[0] * n[1];
+}
+
+// Stages the pairs [row0, row0 + 256) of a cross source into the stage at c.stage. Pairs at or past
+// n_rows read nothing and stage zeros.
+__device__ __forceinline__ void cross_stage(const KParams& P, const WarpCtx& c, int64_t n_rows, uint64_t n_inner) {
+    // one division per tile; a tuple's pair is at most 255 past the tile's first one
+    const uint64_t p0 = (uint64_t)c.row0;
+    const uint64_t o0 = p0 / n_inner, i0 = p0 - o0 * n_inner;
+    uint64_t oi[kR], ii[kR];
+    unsigned ok = 0;
+#pragma unroll
+    for (int r = 0; r < kR; r++) {
+        const uint32_t row = (uint32_t)row_in_tile(r, c.lane);
+        if (n_inner >= (uint64_t)kTile) {
+            ii[r] = i0 + row; oi[r] = o0;
+            if (ii[r] >= n_inner) { ii[r] -= n_inner; oi[r]++; }
+        } else {    // an inner relation of fewer than 256 rows: one tile spans several outer rows
+            const uint32_t d = (uint32_t)i0 + row, q = d / (uint32_t)n_inner;
+            ii[r] = d - q * (uint32_t)n_inner; oi[r] = o0 + q;
+        }
+        if ((int64_t)(p0 + row) < n_rows) ok |= 1u << r;
+    }
+    for (int col = 0; col < P.n_cols; col++) {
+        const int64_t* src = reinterpret_cast<const int64_t*>(P.col_ptr[col]);
+        const bool inner = (P.cross_inner >> col) & 1u;
+        int64_t v[kR];
+#pragma unroll
+        for (int r = 0; r < kR; r++) v[r] = ((ok >> r) & 1) ? __ldg(src + (inner ? ii[r] : oi[r])) : 0;
+        st_m64(c.stage + P.col_off[col] + c.lane * 16, v);
+    }
+    __syncwarp();
+}
+
+template <int GR, bool CROSS = false>
 __global__ void __launch_bounds__(ScanCfg<GR>::kThreads, 1)
 rq_scan_kernel(const __grid_constant__ KParams P) {
+    static_assert(!CROSS || GR == 0, "the cross-source variant has the generic sinks only");
     constexpr int NG = GR > 0 ? GR : 1;                 // register groups
     constexpr int ND = GR > 0 ? GR : kLowCardMaxGroups; // dictionary entries
     // lane / warp-region base are used everywhere; they are made opaque so that the compiler keeps
@@ -307,6 +360,8 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 
     int64_t n_rows = P.n_rows;
     if (P.n_rows_ptr) { n_rows = *P.n_rows_ptr; if (n_rows > P.n_rows_cap) n_rows = P.n_rows_cap; }
+    uint64_t n_inner = 0;
+    if constexpr (CROSS) n_rows = cross_pairs(P, n_inner);
     // tile indices are 32-bit (2^32 tiles = 10^12 rows): cheap to keep or recompute under register pressure
     const uint32_t n_tiles = (uint32_t)((n_rows + kTile - 1) / kTile);
     // a launch may be restricted to the tiles [tile_range[0], tile_range[1]) of the source: the row
@@ -334,7 +389,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(P.insn);
         for (int i = threadIdx.x; i < P.n_insn * 8; i += blockDim.x) sts_b32(prog + i * 4, src[i]);
     }
-    if (lane == 0) {
+    if (!CROSS && lane == 0) {
         for (int s = 0; s < S; s++) mbar_init_s(bars + s * 8, 1);
         fence_mbar_init();
     }
@@ -461,7 +516,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             }
         }
     };
-    if (n_cols > 0) {
+    if (!CROSS && n_cols > 0) {
         for (int s = 0; s < S; s++)
             if ((uint64_t)first + (uint64_t)s * stride < t_end) issue(first + s * stride, s);
     }
@@ -475,7 +530,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         if (hash_sink && *(volatile int32_t*)P.ht_full) {
             // the bulk copies already issued into this warp's stages must land before the CTA may
             // exit (a pending cp.async.bulk into freed shared memory is undefined)
-            if (n_cols > 0) {
+            if (!CROSS && n_cols > 0) {
                 int ds = s;
                 uint32_t dphase = phase;
                 for (int k = 0; k < S; k++) {
@@ -492,7 +547,9 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         c.row0 = (int64_t)tile * (int64_t)kTile;
         c.lane = lane;
 
-        if (n_cols > 0) {
+        if constexpr (CROSS) {
+            if (n_cols > 0) cross_stage(P, c, n_rows, n_inner);
+        } else if (n_cols > 0) {
             if (tile == guarded_tile) {
                 const int64_t rows = n_rows - c.row0;
                 for (int col = 0; col < P.n_cols; col++) {
@@ -510,7 +567,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         // the tile this warp stages next is pulled into L2 while the current one is processed, so
         // the bulk copy issued at the end of the tile is served from L2 (one stage per warp cannot
         // hide the DRAM latency otherwise)
-        if (P.l2_prefetch && elect_one()) {
+        if (!CROSS && P.l2_prefetch && elect_one()) {
             const uint64_t nt = (uint64_t)tile + (uint64_t)S * stride;
             if (nt < t_end && (uint32_t)nt != guarded_tile)
                 for (int c = 0; c < n_runs; c++)
@@ -1348,7 +1405,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         }
         // everyone is done with stage s (and the slots) before it is refilled
         __syncwarp();
-        if (n_cols > 0) {
+        if (!CROSS && n_cols > 0) {
             const uint64_t nt = (uint64_t)tile + (uint64_t)S * stride;
             if (nt < t_end) issue((uint32_t)nt, s);
         }
@@ -1569,17 +1626,6 @@ __global__ void rq_gather_str(const int64_t* addrs, unsigned char* out, int widt
         int k = 0;
         for (; k < width - 1 && s[k] != 0; k++) d[k] = s[k];
         for (; k < width; k++) d[k] = 0;
-    }
-}
-
-// cross product of two materialized relations (NestedLoopsJoinOp): row i = (left i / nr, right i % nr)
-struct CrossCols { const int64_t* in[kMaxStagedCols]; int64_t* out[kMaxStagedCols]; int32_t n_left; int32_t n_right; };
-__global__ void rq_cross_product(CrossCols cc, int64_t nl, int64_t nr) {
-    const int64_t total = nl * nr;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t li = i / nr, ri = i - li * nr;
-        for (int c = 0; c < cc.n_left; c++) cc.out[c][i] = cc.in[c][li];
-        for (int c = 0; c < cc.n_right; c++) cc.out[cc.n_left + c][i] = cc.in[cc.n_left + c][ri];
     }
 }
 
