@@ -74,7 +74,10 @@ void* rq_stream(void);
 /* Engine knobs, the counterpart of the reference's control variables (`threads=4`, `emitmc=true`;
  * processControl, execute.h:454-474). Keys: "split_min_rows", "split_frac" (two-pass probes),
  * "prune_builds", "topk", "replay", "graphs", "direct_joins" (0/1), "stages", "warps" (scan-kernel layout, 0 = automatic),
- * "trace" (0/1). Defaults are the production choices; the parity tests force rarely taken paths. */
+ * "trace" (0/1), "late_materialize" (0 never, 1 = default: materialize pipelines wider than the early form
+ * holds - more than 24 outputs, 16 staged columns, 12 live values or 8 string columns - write row / entry
+ * references and gather their columns afterwards, up to 64 columns; 2: that form wherever it applies).
+ * Defaults are the production choices; the parity tests force rarely taken paths. */
 int rq_set_option(const char* key, double value);
 
 /* Multi-GPU (one process per GPU). rank 0 calls rq_dist_unique_id, the harness broadcasts the

@@ -128,6 +128,7 @@ struct Options {
     bool replay = true;                   // predicted host reads (engine_exec.inl "host reads of device values")
     bool graphs = true;                   // replayed plans are captured into CUDA graphs
     bool zone_skip = true;                // selections on sorted columns restrict the scan to a tile range
+    int late_materialize = 1;             // 0 never, 1 where the early form cannot hold a materialize, 2 wherever it applies
     bool share_builds = true;             // sharded plans: replicated pure-scan builds are split over the ranks and all-reduced
     int64_t share_min_rows = 1 << 20;
     bool narrow = true;                   // host-buffer uploads send 8-byte columns over PCIe in the narrowest exact width
@@ -206,6 +207,8 @@ extern "C" int rq_init(int device) {
         CK(cudaFuncSetAttribute(rq_scan_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         CK(cudaFuncSetAttribute(rq_scan_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         CK(cudaFuncSetAttribute(rq_scan_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+        CK(cudaFuncSetAttribute(rq_scan_kernel<0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+        CK(cudaFuncSetAttribute(rq_scan_kernel<0, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         E.init = true;
         return RQ_OK;
     } catch (RqError& e) {
@@ -257,6 +260,7 @@ extern "C" int rq_set_option(const char* key, double value) {
     else if (k == "graphs") o.graphs = value != 0;
     else if (k == "narrow") o.narrow = value != 0;
     else if (k == "zone_skip") o.zone_skip = value != 0;
+    else if (k == "late_materialize") o.late_materialize = std::max(0, std::min((int)value, 2));
     else if (k == "share_builds") o.share_builds = value != 0;
     else if (k == "share_min_rows") o.share_min_rows = (int64_t)value;
     else if (k == "up_threads") o.up_threads = (int)value;
@@ -785,6 +789,11 @@ struct PipeOut {                    // what a finished pipeline left on the devi
 };
 
 bool is_leaf(int op) { return op == RQ_OP_COL || op == RQ_OP_CONST || op == RQ_OP_CONST_STR; }
+// Nodes only late materialization builds (never accepted from the ABI, run_pipeline checks): the
+// absolute row (pair) index of the tuple, and PAYLOAD with b = kPayloadEntry, the reference of the
+// probe's matched entry (scan kernel variant LATE).
+constexpr int kOpRowId = 1000;
+constexpr int kPayloadEntry = -1;
 bool is_binary(int op) {
     switch (op) {
         case RQ_OP_ADD: case RQ_OP_SUB: case RQ_OP_MUL: case RQ_OP_DIV: case RQ_OP_AND: case RQ_OP_OR:
@@ -868,6 +877,7 @@ struct Lowerer {
     HRef hagg_src[kMaxAggs];
     HRef hprobe_key[kMaxProbes][kMaxKeys];
     int n_slots = 0;
+    int row_slot = -1;                // slot of the kOpRowId node (late materialization)
 
     std::vector<int> uses;            // consumers per node
     std::vector<int> last_use;        // last consuming node index (n = sink)
@@ -973,6 +983,7 @@ struct Lowerer {
                     break;
                 }
                 case RQ_OP_PAYLOAD: check_ref(i, nd.a); break;
+                case kOpRowId: break;
                 default:
                     if (is_binary(nd.op)) { use(i, nd.a); use(i, nd.b); }
                     else raise(RQ_ERR_INVALID, "node %d: unknown op %d", i, nd.op);

@@ -22,6 +22,7 @@ constexpr int kMaxInsn       = 128;
 constexpr int kMaxKeys       = 8;
 constexpr int kMaxAggs       = 16;
 constexpr int kMaxOut        = 24;
+constexpr int kMaxLateOut    = 64;     // output columns of a late-materialized pipeline (IMPL_LATE) and of a result
 constexpr int kMaxImm        = 32;
 constexpr int kMaxProbes     = 4;
 constexpr int kMaxSlots      = 12;
@@ -35,7 +36,8 @@ enum AggMode : uint8_t { AM_FULL = 0, AM_P1 = 1, AM_P2 = 2, AM_W64 = 3 };
 // what the aggregate loop of the register path does for one aggregate (KParams::agg_desc bits 0-2)
 enum AggForm : uint32_t { AF_NONE = 0, AF_P1 = 1, AF_P2 = 2, AF_W64 = 3, AF_FULL = 4, AF_MIN = 5, AF_MAX = 6 };
 
-enum SinkImpl { IMPL_LOWAGG = 1, IMPL_HASHAGG = 2, IMPL_BUILD = 3, IMPL_EMIT = 4, IMPL_REGAGG = 5, IMPL_GROUPJOIN = 6 };
+enum SinkImpl { IMPL_LOWAGG = 1, IMPL_HASHAGG = 2, IMPL_BUILD = 3, IMPL_EMIT = 4, IMPL_REGAGG = 5, IMPL_GROUPJOIN = 6,
+                IMPL_LATE = 7 };   // IMPL_EMIT of a record of references, then rq_late_gather (engine_exec.inl)
 
 // ---- status words of a pipeline launch ----------------------------------------------------------
 // One block in device memory (Engine::flags, 64 bytes) that kernels raise and count into, and its
@@ -289,6 +291,15 @@ struct KParams {
     int64_t        cross_cap[2];         // ... and clamped to the rows each relation has room for
     uint32_t       cross_inner;          // bit c: staged column c belongs to the inner relation
     int32_t        pad3_;
+    // late materialization (kernel variant LATE, engine_exec.inl "late materialization"): before the
+    // program of a tile runs, the absolute row (pair) index of every tuple is written to the slot at
+    // late_row_rel (late_row != 0); probe p writes the reference of its matched entry (hash slot index,
+    // or key - dlo of a direct-address table) to slot late_ref_slot[p] (0xff: none). (Behind every other
+    // field, like the cross fields.)
+    int32_t        late_row;
+    uint32_t       late_row_rel;
+    uint8_t        late_ref_slot[kMaxProbes];
+    int32_t        late;                 // launch the LATE variant
 };
 
 }  // namespace rq

@@ -334,10 +334,15 @@ __device__ __forceinline__ void cross_stage(const KParams& P, const WarpCtx& c, 
     __syncwarp();
 }
 
-template <int GR, bool CROSS = false>
+// LATE (instantiated with GR = 0 only): late materialization. The tile's row (pair) indices go to
+// the slot P.late_row_rel before the program runs, and a probe writes the reference of its matched
+// entry to slot P.late_ref_slot[p]; the materialize sink then writes these references as columns of
+// a record that rq_late_gather resolves into values.
+template <int GR, bool CROSS = false, bool LATE = false>
 __global__ void __launch_bounds__(ScanCfg<GR>::kThreads, 1)
 rq_scan_kernel(const __grid_constant__ KParams P) {
     static_assert(!CROSS || GR == 0, "the cross-source variant has the generic sinks only");
+    static_assert(!LATE || GR == 0, "the late variant has the generic sinks only");
     constexpr int NG = GR > 0 ? GR : 1;                 // register groups
     constexpr int ND = GR > 0 ? GR : kLowCardMaxGroups; // dictionary entries
     // lane / warp-region base are used everywhere; they are made opaque so that the compiler keeps
@@ -581,6 +586,15 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             for (int r = 0; r < kR; r++)
                 if (c.row0 + row_in_tile(r, lane) < n_rows) valid |= 1u << r;
         }
+        if constexpr (LATE) {
+            if (P.late_row) {
+                int64_t rid[kR];
+#pragma unroll
+                for (int r = 0; r < kR; r++) rid[r] = c.row0 + row_in_tile(r, lane);
+                st_m64(wbase + P.late_row_rel + lane * 16, rid);
+                __syncwarp();
+            }
+        }
 
         // ---- 1. the program ---------------------------------------------------------------
         const int n_insn = P.n_insn;
@@ -798,6 +812,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             for (int q = 0; q < pr.n_out; q++)
                                 if (pr.out_slot[q] != 0xff)
                                     sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
+                            if constexpr (LATE) {
+                                if (P.late_ref_slot[in.aux] != 0xff)
+                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, e);
+                            }
                         }
                         __syncwarp();
                         break;
@@ -819,6 +837,14 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             if (!((w[r] >> (idx & 31)) & 1u)) valid &= ~(1u << r);
                         }
                         if (!pr.bloom_only) {
+                            if constexpr (LATE) {
+                                if (P.late_ref_slot[in.aux] != 0xff) {
+                                    const uint32_t dst = wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8);
+#pragma unroll
+                                    for (int r = 0; r < kR; r++)
+                                        sts_b64(dst + row_in_tile(r, lane) * 8, (int64_t)((uint64_t)dk8[r] - (uint64_t)pr.ht.dlo));
+                                }
+                            }
 #pragma unroll 1
                             for (int q = 0; q < pr.n_out; q++) {
                                 if (pr.out_slot[q] == 0xff) continue;
@@ -910,6 +936,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             for (int q = 0; q < pr.n_out; q++)
                                 if (pr.out_slot[q] != 0xff)
                                     sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
+                            if constexpr (LATE) {
+                                if (P.late_ref_slot[in.aux] != 0xff)
+                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, found);
+                            }
                         }
                     } else {
                         unsigned todo = valid;
@@ -942,6 +972,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             for (int q = 0; q < pr.n_out; q++)
                                 if (pr.out_slot[q] != 0xff)
                                     sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
+                            if constexpr (LATE) {
+                                if (P.late_ref_slot[in.aux] != 0xff)
+                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, found);
+                            }
                         }
                     }
                     __syncwarp();
@@ -1626,6 +1660,67 @@ __global__ void rq_gather_str(const int64_t* addrs, unsigned char* out, int widt
         int k = 0;
         for (; k < width - 1 && s[k] != 0; k++) d[k] = s[k];
         for (; k < width; k++) d[k] = 0;
+    }
+}
+
+// Late materialization: fills the deferred output columns of a pipeline from the record its scan
+// wrote (engine_exec.inl "late materialization"). Column k reads its reference from record column
+// ref[k] and resolves it against one source:
+//   LG_ROW    source row r (pair p of a cross source: outer row p / n_inner, inner row p % n_inner)
+//             of a fixed-width column: base + (r / 256) * stride + (r % 256) * width, the page layout
+//             of owned tables (plain arrays have stride = 256 * width); I32 sign-, I8 zero-extended
+//   LG_STR    string column: the address base + r * width, the value the scan's string operand has
+//   LG_HASH   hash-table entry i: ent[i * stride + word]
+//   LG_DIRECT direct-address entry idx: darr[idx * stride + word], or dlo + idx (word < 0: the payload
+//             repeats the key)
+// The record's row count is read on the device and clamped to the output's capacity, so replayed and
+// graph executions need no host read. One thread per (row, column): the writes of a column coalesce.
+enum LateGatherKind : uint8_t { LG_ROW = 0, LG_STR = 1, LG_HASH = 2, LG_DIRECT = 3 };
+struct LateCol {
+    const unsigned char* base;
+    int64_t  stride;        // LG_ROW: bytes per 256-row page; LG_HASH / LG_DIRECT: words per entry
+    int64_t  dlo;
+    int64_t* out;
+    int32_t  word;
+    uint8_t  kind, width, ref, side;    // side (cross source): 0 outer, 1 inner, 2 not a cross source
+};
+struct LateGather {
+    LateCol col[kMaxLateOut];
+    const int64_t* ref[1 + kMaxProbes];
+    const unsigned long long* count;
+    int64_t cap;
+    const int64_t* cross_inner_rows;    // cross source: row count of the inner relation ...
+    int64_t cross_inner_cap;            // ... clamped to its capacity
+};
+__global__ void rq_late_gather(const __grid_constant__ LateGather G) {
+    int64_t n = (int64_t)*G.count;
+    if (n > G.cap) n = G.cap;
+    const LateCol& c = G.col[blockIdx.y];
+    const int64_t* ref = G.ref[c.ref];
+    int64_t n_inner = 1;
+    if (c.side != 2) {
+        n_inner = *G.cross_inner_rows;
+        if (n_inner > G.cross_inner_cap) n_inner = G.cross_inner_cap;
+        if (n_inner < 1) n_inner = 1;
+    }
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t x = ref[i];
+        int64_t v;
+        if (c.kind == LG_HASH) {
+            v = (int64_t)reinterpret_cast<const uint64_t*>(c.base)[(uint64_t)x * (uint64_t)c.stride + c.word];
+        } else if (c.kind == LG_DIRECT) {
+            v = c.word < 0 ? c.dlo + x : (int64_t)reinterpret_cast<const uint64_t*>(c.base)[(uint64_t)x * (uint64_t)c.stride + c.word];
+        } else {
+            const uint64_t r = c.side == 2 ? (uint64_t)x : c.side == 1 ? (uint64_t)x % (uint64_t)n_inner : (uint64_t)x / (uint64_t)n_inner;
+            if (c.kind == LG_STR) {
+                v = (int64_t)(c.base + r * c.width);
+            } else {
+                const unsigned char* a = c.base + (r / kTile) * (uint64_t)c.stride + (r % kTile) * c.width;
+                v = c.width == 8 ? *reinterpret_cast<const int64_t*>(a)
+                  : c.width == 4 ? (int64_t)*reinterpret_cast<const int32_t*>(a) : (int64_t)*a;
+            }
+        }
+        c.out[i] = v;
     }
 }
 
