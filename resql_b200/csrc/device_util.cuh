@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/resql_b200.h"
 #include "rq_internal.h"
 
 namespace rq {
@@ -158,8 +159,8 @@ __device__ __forceinline__ uint64_t mix64(uint64_t h) {
 }
 
 __device__ __forceinline__ int64_t agg_identity(int kind) {
-    if (kind == 3) return INT64_MAX;   // RQ_AGG_MIN
-    if (kind == 4) return INT64_MIN;   // RQ_AGG_MAX
+    if (kind == RQ_AGG_MIN) return INT64_MAX;
+    if (kind == RQ_AGG_MAX) return INT64_MIN;
     return 0;
 }
 

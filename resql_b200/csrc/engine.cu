@@ -203,12 +203,11 @@ extern "C" int rq_init(int device) {
         CK(dmalloc(&E.flags, 64));
         CK(cudaMallocHost(&E.h_flags, 64));
         CK(cudaMallocHost(&E.pinned, 36864));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        CK(cudaFuncSetAttribute(rq_scan_kernel<0, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+        // every kernel scan_kernel_for can return (some more than once)
+        for (int gr : {0, 1, 4})
+            for (bool cross : {false, true})
+                for (bool late : {false, true})
+                    CK(cudaFuncSetAttribute(scan_kernel_for(gr, cross, late), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         E.init = true;
         return RQ_OK;
     } catch (RqError& e) {

@@ -25,10 +25,10 @@ constexpr uint64_t kTagLocked = 1ULL;
 // long runs in a nearly empty table (hashjoin.h:226-256 keeps every duplicate). Walks only give up
 // when somebody raised the table-full flag.
 constexpr uint64_t kFullCheckEvery = 256;
-// flags block of the engine: [0] group overflow, [1] table full, [2] runtime error, [3] long probe run
-// (a claim that had to walk this far: duplicates, or keys clustering under the order-preserving hash)
+// A claim that had to walk this far (duplicates, or keys clustering under the order-preserving hash)
+// raises FlagBlock::dup_key; `full` points at FlagBlock::ht_full (rq_internal.h)
 constexpr uint64_t kLongRun = 1024;
-__device__ __forceinline__ void note_long_run(const int32_t* full) { *const_cast<int32_t*>(full + 2) = 1; }
+__device__ __forceinline__ void note_long_run(const int32_t* full) { *const_cast<int32_t*>(full + kDupKeyFromHtFull) = 1; }
 
 // key kinds: 0 integer word, 1 CHAR (equality ignores trailing blanks), 2 VARCHAR (exact)
 __device__ __forceinline__ uint64_t hash_str(const unsigned char* s, bool strip) {

@@ -11,6 +11,12 @@
 //   2. runs the sink as straight-line code: group match + aggregation, hash aggregation,
 //      hash-join build, or materialize;
 //   3. re-arms the stage. No CTA-wide barrier exists in the steady state.
+// Staging is done by named pieces: issue_tile (the bulk copies of one stage), stage_tile (wait, or
+// stage the guarded tail of a borrowed source, or the pairs of a cross source), prefetch_next (L2
+// prefetch of the next tile) and drain_ring (early exit on a full hash table). Repeated sink pieces
+// have one definition each: atomic_agg (hash aggregation and groupjoin), put_match (probe matches),
+// warp_group_slot (group-table slot of a flush), leader_key (a new dictionary key), reg_at / reg_set
+// (an element of a register array).
 //
 // Aggregation (template parameter GR):
 //   GR = 1 / 4  register path: up to GR groups x kNAR aggregates live in registers for the whole
@@ -27,6 +33,7 @@
 //   string compares        src/qlib/scalar.h:16-120
 #pragma once
 #include <cuda_runtime.h>
+#include "../../include/resql_b200.h"
 #include "rq_internal.h"
 #include "device_util.cuh"
 #include "hash_kernels.cuh"
@@ -207,18 +214,19 @@ __device__ __forceinline__ void pack_keys(const KParams& P, const WarpCtx& c, ui
     }
 }
 
-// acc += (low word of v) * m : IMAD.WIDE.U32 with 64-bit accumulate, one FMA-pipe instruction
-__device__ __forceinline__ void mad_wide_u32(uint64_t& acc, uint32_t a, uint32_t m) {
-    asm("mad.wide.u32 %0, %1, %2, %0;" : "+l"(acc) : "r"(a), "r"(m));
+// element i of a register array, and setting it: one compare-select per element keeps the array in
+// registers, where a dynamic index would move it to local memory
+template <typename T, int N>
+__device__ __forceinline__ T reg_at(const T (&a)[N], int i) {
+    T x = 0;
+#pragma unroll
+    for (int q = 0; q < N; q++) if (q == i) x = a[q];
+    return x;
 }
-// acc += (signed high word of v) * m : IMAD.WIDE (signed) with 64-bit accumulate
-__device__ __forceinline__ void mad_wide_s32(int64_t& acc, int32_t a, int32_t m) {
-    asm("mad.wide.s32 %0, %1, %2, %0;" : "+l"(acc) : "r"(a), "r"(m));
-}
-
-// acc.hi += a * m (low 32 bits of the product): the high-word half of acc += (a << 32) * m
-__device__ __forceinline__ void mad_hi_word(uint64_t& acc, uint32_t a, uint32_t m) {
-    asm("{\n.reg .u32 lo, hi;\nmov.b64 {lo, hi}, %0;\nmad.lo.u32 hi, %1, %2, hi;\nmov.b64 %0, {lo, hi};\n}" : "+l"(acc) : "r"(a), "r"(m));
+template <typename T, int N>
+__device__ __forceinline__ void reg_set(T (&a)[N], int i, T x) {
+#pragma unroll
+    for (int q = 0; q < N; q++) if (q == i) a[q] = x;
 }
 
 // ---- low-cardinality global group table (packed key) -----------------------------------------
@@ -240,13 +248,23 @@ __device__ __forceinline__ int group_table_slot(const KParams& P, uint64_t key) 
     }
     return -1;
 }
+// the same for a whole warp: lane 0 looks the key up (with nk = 0 grouping keys, the one key 0) and
+// raises the overflow flag when the table is full; every lane gets the slot (-1: full)
+__device__ __forceinline__ int warp_group_slot(const KParams& P, int nk, uint64_t key, int lane) {
+    int slot = -1;
+    if (lane == 0) {
+        slot = group_table_slot(P, nk == 0 ? 0ULL : key);
+        if (slot < 0) *P.overflow = 1;
+    }
+    return __shfl_sync(kFull, slot, 0);
+}
 
 __device__ __forceinline__ int64_t warp_reduce(int64_t v, int kind) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         const int64_t w = __shfl_xor_sync(kFull, v, o);
-        if (kind == 3) v = w < v ? w : v;
-        else if (kind == 4) v = w > v ? w : v;
+        if (kind == RQ_AGG_MIN) v = w < v ? w : v;
+        else if (kind == RQ_AGG_MAX) v = w > v ? w : v;
         else v = (int64_t)((uint64_t)v + (uint64_t)w);
     }
     return v;
@@ -254,9 +272,42 @@ __device__ __forceinline__ int64_t warp_reduce(int64_t v, int kind) {
 
 __device__ __forceinline__ void group_table_add(const KParams& P, int slot, int a, int kind, int64_t v) {
     int64_t* dst = &P.g_acc[(size_t)slot * kMaxAggs + a];
-    if (kind == 3) atomicMin((long long*)dst, (long long)v);
-    else if (kind == 4) atomicMax((long long*)dst, (long long)v);
+    if (kind == RQ_AGG_MIN) atomicMin((long long*)dst, (long long)v);
+    else if (kind == RQ_AGG_MAX) atomicMax((long long*)dst, (long long)v);
     else atomicAdd((unsigned long long*)dst, (unsigned long long)v);
+}
+
+// adds tuple r to aggregate a, whose word is acc[a] (hash aggregation and groupjoin entries)
+__device__ __forceinline__ void atomic_agg(const KParams& P, const WarpCtx& c, uint64_t* acc, int a, int r) {
+    const int kind = P.agg_kind[a];
+    if (kind == RQ_AGG_COUNT) { atomicAdd((unsigned long long*)&acc[a], 1ULL); return; }
+    const int64_t v = ld_row(P, c, P.agg_src[a], r);
+    if (kind == RQ_AGG_SUM) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
+    else if (kind == RQ_AGG_MIN) atomicMin((long long*)&acc[a], (long long)v);
+    else atomicMax((long long*)&acc[a], (long long)v);
+}
+
+// group match: the key of the first unmatched tuple (bit of `unk`) of the lowest lane that has one,
+// on every lane
+__device__ __forceinline__ uint64_t leader_key(unsigned unk, const uint64_t (&key)[kR]) {
+    const unsigned ball = __ballot_sync(kFull, unk != 0);
+    const int leader = __ffs(ball) - 1;
+    const uint64_t lk = reg_at(key, __ffs(unk) - 1);
+    return __shfl_sync(kFull, lk, leader);
+}
+
+// a probe match of the tuple at `row`: the entry's payload words go to their value slots and, in the
+// late variant, the entry reference `ref` to the probe's reference slot
+template <bool LATE>
+__device__ __forceinline__ void put_match(const KParams& P, const DProbe& pr, int p, uint32_t wbase, int row,
+                                          const uint64_t* ent, int64_t ref) {
+    for (int q = 0; q < pr.n_out; q++)
+        if (pr.out_slot[q] != 0xff)
+            sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
+    if constexpr (LATE) {
+        if (P.late_ref_slot[p] != 0xff)
+            sts_b64(wbase + P.slots_rel + P.late_ref_slot[p] * (kTile * 8) + row * 8, ref);
+    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -276,11 +327,6 @@ extern __shared__ __align__(128) unsigned char rq_smem[];
 #define RQ_EX_GE(x, y)   ((int64_t)((x) >= (y)))
 #define RQ_EX_EQ(x, y)   ((int64_t)((x) == (y)))
 #define RQ_EX_NE(x, y)   ((int64_t)((x) != (y)))
-
-template <int GR> struct ScanCfg;
-template <> struct ScanCfg<0> { static constexpr int kThreads = 512; };
-template <> struct ScanCfg<1> { static constexpr int kThreads = 512; };
-template <> struct ScanCfg<4> { static constexpr int kThreads = 512; };
 
 // Nested-loops join source (CROSS, instantiated with GR = 0 only): the pairs of two relations are
 // never materialized. Tile t holds pairs [256t, 256t + 256); pair p is (outer row p / n_inner, inner
@@ -334,12 +380,93 @@ __device__ __forceinline__ void cross_stage(const KParams& P, const WarpCtx& c, 
     __syncwarp();
 }
 
+// ---- staging ----------------------------------------------------------------------------------
+// A warp's ring of S stages and the tiles it walks: first, first + stride, ... below t_end.
+struct Ring {
+    uint32_t bars;          // shared address of the warp's mbarriers, one per stage
+    uint32_t wbase;         // shared address of the warp's region; stage s is at wbase + s * P.stage_bytes
+    int      S;
+    uint32_t stride, t_end;
+    uint32_t guarded_tile;  // the partial last tile of a borrowed source (0xffffffff: none)
+    uint64_t policy;        // L2 policy of the bulk copies
+    int      n_runs;
+    bool     hint;          // copy with the L2 policy
+};
+
+// One lane issues the bulk copies of all staged columns of a tile into stage s (uniform operands)
+// after arming the stage's barrier with its byte count. The guarded tile is staged by plain loads.
+__device__ __forceinline__ void issue_tile(const KParams& P, const Ring& g, uint32_t tile, int s) {
+    if (tile == g.guarded_tile) return;
+    if (elect_one()) {
+        const uint32_t bar = g.bars + s * 8;
+        const uint32_t dst0 = g.wbase + s * P.stage_bytes;
+        const uint32_t t32 = tile;
+        mbar_expect_tx_s(bar, P.stage_bytes);
+        if (g.hint) {
+            for (int c = 0; c < g.n_runs; c++)
+                tma_bulk_g2s_hint(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar, g.policy);
+        } else {
+            for (int c = 0; c < g.n_runs; c++)
+                tma_bulk_g2s_s(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar);
+        }
+    }
+}
+
+// Early exit on a full hash table: the bulk copies already issued into this warp's stages (tiles
+// `tile` onwards, starting at stage s) must land before the CTA may exit (a pending cp.async.bulk
+// into freed shared memory is undefined).
+__device__ __forceinline__ void drain_ring(const Ring& g, uint32_t tile, int s, uint32_t phase) {
+    int ds = s;
+    uint32_t dphase = phase;
+    for (int k = 0; k < g.S; k++) {
+        const uint64_t t = (uint64_t)tile + (uint64_t)k * g.stride;
+        if (t < g.t_end && (uint32_t)t != g.guarded_tile) mbar_wait_s(g.bars + ds * 8, dphase);
+        if (++ds == g.S) { ds = 0; dphase ^= 1u; }
+    }
+}
+
+// The tile at c.row0 is in stage s after this: the bulk copies have landed, or the guarded tail of
+// a borrowed source was staged with plain loads (zeros past n_rows), or the warp staged the pairs of
+// a cross source itself.
+template <bool CROSS>
+__device__ __forceinline__ void stage_tile(const KParams& P, const WarpCtx& c, const Ring& g, uint32_t tile, int s,
+                                           uint32_t phase, int64_t n_rows, uint64_t n_inner, int n_cols) {
+    if constexpr (CROSS) {
+        if (n_cols > 0) cross_stage(P, c, n_rows, n_inner);
+    } else if (n_cols > 0) {
+        if (tile == g.guarded_tile) {
+            const int64_t rows = n_rows - c.row0;
+            for (int col = 0; col < P.n_cols; col++) {
+                const int w = P.col_w[col];
+                const unsigned char* src = P.col_ptr[col] + (size_t)c.row0 * w;
+                for (int i = c.lane; i < kTile * w; i += 32)
+                    sts_u8(c.stage + P.col_off[col] + i, (i < rows * w) ? src[i] : 0u);
+            }
+            __syncwarp();
+        } else {
+            mbar_wait_s(g.bars + s * 8, phase);
+        }
+    }
+}
+
+// The tile this warp stages next is pulled into L2 while the current one is processed, so the bulk
+// copy issued at the end of the tile is served from L2 (one stage per warp cannot hide the DRAM
+// latency otherwise).
+__device__ __forceinline__ void prefetch_next(const KParams& P, const Ring& g, uint32_t tile) {
+    if (P.l2_prefetch && elect_one()) {
+        const uint64_t nt = (uint64_t)tile + (uint64_t)g.S * g.stride;
+        if (nt < g.t_end && (uint32_t)nt != g.guarded_tile)
+            for (int c = 0; c < g.n_runs; c++)
+                tma_prefetch_l2(P.run_ptr[c] + (size_t)(uint32_t)nt * P.run_stride[c], P.run_bytes[c]);
+    }
+}
+
 // LATE (instantiated with GR = 0 only): late materialization. The tile's row (pair) indices go to
 // the slot P.late_row_rel before the program runs, and a probe writes the reference of its matched
 // entry to slot P.late_ref_slot[p]; the materialize sink then writes these references as columns of
 // a record that rq_late_gather resolves into values.
 template <int GR, bool CROSS = false, bool LATE = false>
-__global__ void __launch_bounds__(ScanCfg<GR>::kThreads, 1)
+__global__ void __launch_bounds__(kMaxWarps * 32, 1)
 rq_scan_kernel(const __grid_constant__ KParams P) {
     static_assert(!CROSS || GR == 0, "the cross-source variant has the generic sinks only");
     static_assert(!LATE || GR == 0, "the late variant has the generic sinks only");
@@ -431,21 +558,16 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll
         for (int g = 0; g < NG; g++) {
             if (g >= n) continue;
-            int slot = -1;
-            if (lane == 0) {
-                slot = group_table_slot(P, NK == 0 ? 0ULL : dk[g]);
-                if (slot < 0) *P.overflow = 1;
-            }
-            slot = __shfl_sync(kFull, slot, 0);
+            const int slot = warp_group_slot(P, NK, dk[g], lane);
 #pragma unroll
             for (int a = 0; a < kNAR; a++) {
                 if (a >= NA) continue;
                 const int kind = P.agg_kind[a];
                 const int mode = P.agg_mode[a];
                 uint64_t part;
-                if (kind == 2) part = rcnt[g];
-                else if (kind == 1 && mode == AM_P1) part = racc[g][2 * a];
-                else if (kind == 1 && mode == AM_P2) part = (uint64_t)racc[g][2 * a] + ((uint64_t)racc[g][2 * a + 1] << P.agg_shift[a]);
+                if (kind == RQ_AGG_COUNT) part = rcnt[g];
+                else if (kind == RQ_AGG_SUM && mode == AM_P1) part = racc[g][2 * a];
+                else if (kind == RQ_AGG_SUM && mode == AM_P2) part = (uint64_t)racc[g][2 * a] + ((uint64_t)racc[g][2 * a + 1] << P.agg_shift[a]);
                 else part = (uint64_t)racc[g][2 * a] | ((uint64_t)racc[g][2 * a + 1] << 32);
                 const int64_t v = warp_reduce((int64_t)part, kind);
                 if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, v);
@@ -467,21 +589,16 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll
         for (int g = 0; g < NG; g++) {
             if (g >= n) continue;
-            int slot = -1;
-            if (lane == 0) {
-                slot = group_table_slot(P, NK == 0 ? 0ULL : dk[g]);
-                if (slot < 0) *P.overflow = 1;
-            }
-            slot = __shfl_sync(kFull, slot, 0);
+            const int slot = warp_group_slot(P, NK, dk[g], lane);
 #pragma unroll
             for (int a = 0; a < kNAR; a++) {
                 if (a >= NA) continue;
                 const int kind = P.agg_kind[a];
                 const int mode = P.agg_mode[a];
                 uint64_t part;
-                if (kind == 2) part = warp_sum_u32(rcnt[g]);
-                else if (kind == 1 && mode == AM_P1) { part = warp_sum_u32(racc[g][2 * a]); racc[g][2 * a] = 0; }
-                else if (kind == 1 && mode == AM_P2) {
+                if (kind == RQ_AGG_COUNT) part = warp_sum_u32(rcnt[g]);
+                else if (kind == RQ_AGG_SUM && mode == AM_P1) { part = warp_sum_u32(racc[g][2 * a]); racc[g][2 * a] = 0; }
+                else if (kind == RQ_AGG_SUM && mode == AM_P2) {
                     part = warp_sum_u32(racc[g][2 * a]) + (warp_sum_u32(racc[g][2 * a + 1]) << P.agg_shift[a]);
                     racc[g][2 * a] = 0; racc[g][2 * a + 1] = 0;
                 } else continue;
@@ -496,34 +613,15 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     }
     __syncwarp();
 
-    // a partial last tile of a borrowed (unpadded) source is staged with guarded plain loads
-    const uint32_t guarded_tile = (P.borrowed && ((uint32_t)n_rows & (kTile - 1)) != 0) ? n_tiles - 1 : 0xffffffffu;
-    // One lane issues the bulk copies of all staged columns of a tile (uniform operands) after arming
-    // the barrier with the stage's byte count. Scanned data is streamed once, so it is marked
-    // evict-first in L2.
-    const uint64_t stream_policy = l2_evict_first_policy();
+    // a partial last tile of a borrowed (unpadded) source is staged with guarded plain loads;
+    // scanned data is streamed once, so it is marked evict-first in L2
+    const Ring ring{bars, wbase, S, stride, t_end,
+                    (P.borrowed && ((uint32_t)n_rows & (kTile - 1)) != 0) ? n_tiles - 1 : 0xffffffffu,
+                    l2_evict_first_policy(), P.n_runs, P.stream_hint != 0};
     const int n_cols = P.n_cols;
-    const int n_runs = P.n_runs;
-    const bool hint = P.stream_hint != 0;
-    auto issue = [&](uint32_t tile, int s) {
-        if (tile == guarded_tile) return;
-        if (elect_one()) {
-            const uint32_t bar = bars + s * 8;
-            const uint32_t dst0 = wbase + s * P.stage_bytes;
-            const uint32_t t32 = tile;
-            mbar_expect_tx_s(bar, P.stage_bytes);
-            if (hint) {
-                for (int c = 0; c < n_runs; c++)
-                    tma_bulk_g2s_hint(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar, stream_policy);
-            } else {
-                for (int c = 0; c < n_runs; c++)
-                    tma_bulk_g2s_s(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar);
-            }
-        }
-    };
     if (!CROSS && n_cols > 0) {
         for (int s = 0; s < S; s++)
-            if ((uint64_t)first + (uint64_t)s * stride < t_end) issue(first + s * stride, s);
+            if ((uint64_t)first + (uint64_t)s * stride < t_end) issue_tile(P, ring, first + s * stride, s);
     }
 
     int s = 0;
@@ -533,17 +631,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     for (uint32_t tile = first; tile < t_end; tile += stride) {
         // a full hash table makes the host regrow it and rerun: stop early
         if (hash_sink && *(volatile int32_t*)P.ht_full) {
-            // the bulk copies already issued into this warp's stages must land before the CTA may
-            // exit (a pending cp.async.bulk into freed shared memory is undefined)
-            if (!CROSS && n_cols > 0) {
-                int ds = s;
-                uint32_t dphase = phase;
-                for (int k = 0; k < S; k++) {
-                    const uint64_t t = (uint64_t)tile + (uint64_t)k * stride;
-                    if (t < t_end && (uint32_t)t != guarded_tile) mbar_wait_s(bars + ds * 8, dphase);
-                    if (++ds == S) { ds = 0; dphase ^= 1u; }
-                }
-            }
+            if (!CROSS && n_cols > 0) drain_ring(ring, tile, s, phase);
             break;
         }
         WarpCtx c;
@@ -552,32 +640,8 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         c.row0 = (int64_t)tile * (int64_t)kTile;
         c.lane = lane;
 
-        if constexpr (CROSS) {
-            if (n_cols > 0) cross_stage(P, c, n_rows, n_inner);
-        } else if (n_cols > 0) {
-            if (tile == guarded_tile) {
-                const int64_t rows = n_rows - c.row0;
-                for (int col = 0; col < P.n_cols; col++) {
-                    const int w = P.col_w[col];
-                    const unsigned char* src = P.col_ptr[col] + (size_t)c.row0 * w;
-                    for (int i = lane; i < kTile * w; i += 32)
-                        sts_u8(c.stage + P.col_off[col] + i, (i < rows * w) ? src[i] : 0u);
-                }
-                __syncwarp();
-            } else {
-                mbar_wait_s(bars + s * 8, phase);
-            }
-        }
-
-        // the tile this warp stages next is pulled into L2 while the current one is processed, so
-        // the bulk copy issued at the end of the tile is served from L2 (one stage per warp cannot
-        // hide the DRAM latency otherwise)
-        if (!CROSS && P.l2_prefetch && elect_one()) {
-            const uint64_t nt = (uint64_t)tile + (uint64_t)S * stride;
-            if (nt < t_end && (uint32_t)nt != guarded_tile)
-                for (int c = 0; c < n_runs; c++)
-                    tma_prefetch_l2(P.run_ptr[c] + (size_t)(uint32_t)nt * P.run_stride[c], P.run_bytes[c]);
-        }
+        stage_tile<CROSS>(P, c, ring, tile, s, phase, n_rows, n_inner, n_cols);
+        if (!CROSS) prefetch_next(P, ring, tile);
 
         unsigned valid = 0xffu;
         if (c.row0 + kTile > n_rows) {
@@ -804,18 +868,8 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll 1
                         for (int r = 0; r < kR; r++) {
                             if (!((valid >> r) & 1)) continue;
-                            int64_t e = 0;
-#pragma unroll
-                            for (int q = 0; q < kR; q++) if (q == r) e = ei[q];
-                            const uint64_t* ent = ht_entry(pr.ht, (uint64_t)e);
-                            const int row = row_in_tile(r, lane);
-                            for (int q = 0; q < pr.n_out; q++)
-                                if (pr.out_slot[q] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
-                            if constexpr (LATE) {
-                                if (P.late_ref_slot[in.aux] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, e);
-                            }
+                            const int64_t e = reg_at(ei, r);
+                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)e), e);
                         }
                         __syncwarp();
                         break;
@@ -882,9 +936,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             if (!((valid >> r) & 1)) continue;
                             int64_t k[kMaxKeys];
                             for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, pr.key[j], r);
-                            const uint64_t hv = hash_typed(k, pr.ht.key_kind, pnk);
-#pragma unroll
-                            for (int q = 0; q < kR; q++) if (q == r) h[q] = hv;
+                            reg_set(h, r, hash_typed(k, pr.ht.key_kind, pnk));
                         }
                     }
                     if (pr.ht.bloom != nullptr) {
@@ -931,24 +983,14 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             }
                             if (found < 0) { valid &= ~(1u << r); continue; }
                             if (matches > 1) atomicAdd(pr.dup_counter, (unsigned long long)(matches - 1));
-                            const int row = row_in_tile(r, lane);
-                            const uint64_t* ent = ht_entry(pr.ht, (uint64_t)found);
-                            for (int q = 0; q < pr.n_out; q++)
-                                if (pr.out_slot[q] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
-                            if constexpr (LATE) {
-                                if (P.late_ref_slot[in.aux] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, found);
-                            }
+                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
                         }
                     } else {
                         unsigned todo = valid;
                         while (todo) {
                             const int r = __ffs(todo) - 1;
                             todo &= todo - 1;
-                            uint64_t hr = 0;
-#pragma unroll
-                            for (int q = 0; q < kR; q++) if (q == r) hr = h[q];
+                            const uint64_t hr = reg_at(h, r);
                             int64_t k[kMaxKeys];
                             for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, pr.key[j], r);
                             const uint64_t tag = hr | 2ULL;
@@ -967,15 +1009,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             }
                             if (found < 0) { valid &= ~(1u << r); continue; }
                             if (matches > 1) atomicAdd(pr.dup_counter, (unsigned long long)(matches - 1));
-                            const int row = row_in_tile(r, lane);
-                            const uint64_t* ent = ht_entry(pr.ht, (uint64_t)found);
-                            for (int q = 0; q < pr.n_out; q++)
-                                if (pr.out_slot[q] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
-                            if constexpr (LATE) {
-                                if (P.late_ref_slot[in.aux] != 0xff)
-                                    sts_b64(wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8) + row * 8, found);
-                            }
+                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
                         }
                     }
                     __syncwarp();
@@ -1058,13 +1092,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             for (int g = 0; g < NG; g++) any |= m[g][r];
                             if ((valid & (1u << r)) && any == 0) unk |= 1u << r;
                         }
-                        const unsigned ball = __ballot_sync(kFull, unk != 0);
-                        const int leader = __ffs(ball) - 1;
-                        uint64_t lk = 0;
-                        const int rr = __ffs(unk) - 1;
-#pragma unroll
-                        for (int r = 0; r < kR; r++) if (r == rr) lk = key[r];
-                        lk = __shfl_sync(kFull, lk, leader);
+                        const uint64_t lk = leader_key(unk, key);
                         if (ngroups >= NG) {
                             // more groups than this path tracks: the host reruns with the next
                             // implementation; the unmatched tuples are simply dropped here
@@ -1074,8 +1102,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             for (int g = 0; g < NG; g++) rcnt[g] += ct[g];
                             break;
                         }
-#pragma unroll
-                        for (int e = 0; e < NG; e++) if (e == ngroups) dk[e] = lk;
+                        reg_set(dk, ngroups, lk);
                         ngroups++;
                     }
                 }
@@ -1102,7 +1129,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     int64_t v[kR];
                     if (desc & 8u) ld_m64(((desc & 16u) ? c.wbase : c.stage) + (desc >> 8) + lane * 16, v);
                     else fetch_vref(P, c, P.agg_src[a], v);
-                    const int kind = form == AF_MIN ? 3 : 4;
+                    const int kind = form == AF_MIN ? RQ_AGG_MIN : RQ_AGG_MAX;
                     if (form == AF_P1) {
 #pragma unroll
                         for (int r = 0; r < kR; r++)
@@ -1146,7 +1173,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             int64_t best = (int64_t)((uint64_t)racc[g][2 * a] | ((uint64_t)racc[g][2 * a + 1] << 32));
 #pragma unroll
                             for (int r = 0; r < kR; r++)
-                                if (m[g][r] && (kind == 3 ? v[r] < best : v[r] > best)) best = v[r];
+                                if (m[g][r] && (kind == RQ_AGG_MIN ? v[r] < best : v[r] > best)) best = v[r];
                             racc[g][2 * a] = (uint32_t)(uint64_t)best; racc[g][2 * a + 1] = (uint32_t)((uint64_t)best >> 32);
                         }
                     }
@@ -1171,20 +1198,13 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         gid |= g << (4 * r);
                     }
                     while (__any_sync(kFull, unk != 0)) {
-                        const unsigned ball = __ballot_sync(kFull, unk != 0);
-                        const int leader = __ffs(ball) - 1;
-                        uint64_t lk = 0;
-                        const int rr = __ffs(unk) - 1;
-#pragma unroll
-                        for (int r = 0; r < kR; r++) if (r == rr) lk = key[r];
-                        lk = __shfl_sync(kFull, lk, leader);
+                        const uint64_t lk = leader_key(unk, key);
                         if (ngroups >= P.G) {
                             if (lane == 0) *P.overflow = 1;
                             unk = 0;
                             break;
                         }
-#pragma unroll
-                        for (int e = 0; e < ND; e++) if (e == ngroups) dk[e] = lk;
+                        reg_set(dk, ngroups, lk);
 #pragma unroll
                         for (int r = 0; r < kR; r++) {
                             if (((unk >> r) & 1) && key[r] == lk) {
@@ -1198,7 +1218,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                 for (int a = 0; a < NA; a++) {
                     const int kind = P.agg_kind[a];
                     int64_t v[kR];
-                    if (kind != 2) fetch_vref(P, c, P.agg_src[a], v);
+                    if (kind != RQ_AGG_COUNT) fetch_vref(P, c, P.agg_src[a], v);
                     const uint32_t base = sacc + (a * 32 + lane) * 8;
 #pragma unroll
                     for (int r = 0; r < kR; r++) {
@@ -1206,9 +1226,9 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             const uint32_t p = base + ((gid >> (4 * r)) & 15) * NA * 256;
                             const int64_t cur = lds_b64(p);
                             int64_t nv;
-                            if (kind == 2) nv = cur + 1;
-                            else if (kind == 1) nv = (int64_t)((uint64_t)cur + (uint64_t)v[r]);
-                            else if (kind == 3) nv = v[r] < cur ? v[r] : cur;
+                            if (kind == RQ_AGG_COUNT) nv = cur + 1;
+                            else if (kind == RQ_AGG_SUM) nv = (int64_t)((uint64_t)cur + (uint64_t)v[r]);
+                            else if (kind == RQ_AGG_MIN) nv = v[r] < cur ? v[r] : cur;
                             else nv = v[r] > cur ? v[r] : cur;
                             sts_b64(p, nv);
                         }
@@ -1315,14 +1335,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     if (!ok) { *P.ht_full = 1; continue; }
                     if (cur == 0ULL) n_inserted++;
                     uint64_t* acc = ht_entry(P.ht, slot) + 1;
-                    for (int a = 0; a < NA; a++) {
-                        const int kind = P.agg_kind[a];
-                        if (kind == 2) { atomicAdd((unsigned long long*)&acc[a], 1ULL); continue; }
-                        const int64_t v = ld_row(P, c, P.agg_src[a], r);
-                        if (kind == 1) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
-                        else if (kind == 3) atomicMin((long long*)&acc[a], (long long)v);
-                        else atomicMax((long long*)&acc[a], (long long)v);
-                    }
+                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
                 }
             } else if (sink == IMPL_HASHAGG) {
                 for (unsigned todo = valid; todo; todo &= todo - 1) {
@@ -1335,14 +1348,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     if (!ht_find_or_insert(P.ht, k, hh, &slot, &fresh, P.ht_full)) { *P.ht_full = 1; continue; }
                     if (fresh) n_inserted++;
                     uint64_t* acc = ht_entry(P.ht, slot) + 1 + P.ht.nk;
-                    for (int a = 0; a < NA; a++) {
-                        const int kind = P.agg_kind[a];
-                        if (kind == 2) { atomicAdd((unsigned long long*)&acc[a], 1ULL); continue; }
-                        const int64_t v = ld_row(P, c, P.agg_src[a], r);
-                        if (kind == 1) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
-                        else if (kind == 3) atomicMin((long long*)&acc[a], (long long)v);
-                        else atomicMax((long long*)&acc[a], (long long)v);
-                    }
+                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
                 }
             } else if (sink == IMPL_GROUPJOIN) {
                 // GROUP BY on the key of a direct-address join (engine_exec.inl groupjoin_probe): the
@@ -1355,20 +1361,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll 1
                 for (int r = 0; r < kR; r++) {
                     if (!((valid >> r) & 1)) continue;
-                    int64_t k = 0;
-#pragma unroll
-                    for (int q = 0; q < kR; q++) if (q == r) k = gk[q];
-                    const uint64_t idx = (uint64_t)k - (uint64_t)P.ht.dlo;
+                    const uint64_t idx = (uint64_t)reg_at(gk, r) - (uint64_t)P.ht.dlo;
                     atomicOr(&P.gj_touched[idx >> 5], 1u << (idx & 31));
                     uint64_t* acc = P.ht.darr + idx * P.ht.dnv + P.gj_acc_word;
-                    for (int a = 0; a < NA; a++) {
-                        const int kind = P.agg_kind[a];
-                        if (kind == 2) { atomicAdd((unsigned long long*)&acc[a], 1ULL); continue; }
-                        const int64_t v = ld_row(P, c, P.agg_src[a], r);
-                        if (kind == 1) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
-                        else if (kind == 3) atomicMin((long long*)&acc[a], (long long)v);
-                        else atomicMax((long long*)&acc[a], (long long)v);
-                    }
+                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
                 }
             } else if (sink == IMPL_EMIT && P.expand_probe >= 0) {
                 // multi-match hash join (hashjoin.h:118-165): one output row per key-equal entry.
@@ -1441,7 +1437,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         __syncwarp();
         if (!CROSS && n_cols > 0) {
             const uint64_t nt = (uint64_t)tile + (uint64_t)S * stride;
-            if (nt < t_end) issue((uint32_t)nt, s);
+            if (nt < t_end) issue_tile(P, ring, (uint32_t)nt, s);
         }
         if (++s == S) { s = 0; phase ^= 1u; }
         if (GR > 0 && P.flush_tiles > 0 && --tiles_to_flush == 0) {
@@ -1460,15 +1456,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         } else {
             if (n > P.G) n = P.G;
             for (int e = 0; e < n; e++) {
-                uint64_t kk = 0;
-#pragma unroll
-                for (int q = 0; q < ND; q++) if (q == e) kk = dk[q];
-                int slot = -1;
-                if (lane == 0) {
-                    slot = group_table_slot(P, NK == 0 ? 0ULL : kk);
-                    if (slot < 0) *P.overflow = 1;
-                }
-                slot = __shfl_sync(kFull, slot, 0);
+                const int slot = warp_group_slot(P, NK, reg_at(dk, e), lane);
                 for (int a = 0; a < NA; a++) {
                     const int kind = P.agg_kind[a];
                     const int64_t v = warp_reduce(lds_b64(sacc + ((e * NA + a) * 32 + lane) * 8), kind);
@@ -1477,6 +1465,15 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             }
         }
     }
+}
+
+// The instantiations of the scan kernel and the one a launch uses: gr is the number of register
+// groups (0, 1 or 4); the cross-source and late variants exist for gr = 0 only and take precedence.
+using ScanKernel = void (*)(KParams);
+inline ScanKernel scan_kernel_for(int gr, bool cross, bool late) {
+    if (late) return cross ? rq_scan_kernel<0, true, true> : rq_scan_kernel<0, false, true>;
+    if (cross) return rq_scan_kernel<0, true>;
+    return gr == 4 ? rq_scan_kernel<4> : gr == 1 ? rq_scan_kernel<1> : rq_scan_kernel<0>;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1592,7 +1589,7 @@ __global__ void rq_sorted_tile_range(const unsigned char* col, int width, int64_
 __global__ void rq_popcount_words(const uint32_t* w, size_t n, unsigned long long* out) {
     unsigned long long c = 0;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) c += __popc(w[i]);
-    c = (unsigned long long)warp_reduce((int64_t)c, 1);
+    c = (unsigned long long)warp_reduce((int64_t)c, RQ_AGG_SUM);
     if ((threadIdx.x & 31) == 0 && c) atomicAdd(out, c);
 }
 // ... must equal the summed entry count (FlagBlock::entries), else two ranks inserted the same key:
@@ -1618,8 +1615,8 @@ __global__ void rq_col_minmax(const unsigned char* col, int width, int64_t tile_
         lo = v < lo ? v : lo;
         hi = v > hi ? v : hi;
     }
-    lo = warp_reduce(lo, 3);
-    hi = warp_reduce(hi, 4);
+    lo = warp_reduce(lo, RQ_AGG_MIN);
+    hi = warp_reduce(hi, RQ_AGG_MAX);
     if ((threadIdx.x & 31) == 0) {
         atomicMin((long long*)&out[0], (long long)lo);
         atomicMax((long long*)&out[1], (long long)hi);
