@@ -76,7 +76,10 @@ void* rq_stream(void);
  * "prune_builds", "topk", "replay", "graphs", "direct_joins" (0/1), "stages", "warps" (scan-kernel layout, 0 = automatic),
  * "trace" (0/1), "late_materialize" (0 never, 1 = default: materialize pipelines wider than the early form
  * holds - more than 24 outputs, 16 staged columns, 12 live values or 8 string columns - write row / entry
- * references and gather their columns afterwards, up to 64 columns; 2: that form wherever it applies).
+ * references and gather their columns afterwards, up to 64 columns; 2: that form wherever it applies),
+ * "in_lists" (OR trees of equality tests of one value against constants as one set test: 0 never, keeping
+ * one compare per value; 1 = default: integer lists of 2 values or more, string lists of 4 or more;
+ * 2: every list of 2 values or more).
  * Defaults are the production choices; the parity tests force rarely taken paths. */
 int rq_set_option(const char* key, double value);
 
@@ -151,7 +154,10 @@ enum rq_op {
     RQ_OP_MUL,          /* a * b   low 64 bits (imul)                   (:371-402)             */
     RQ_OP_DIV,          /* a / b   truncating (cqo; idiv)               (:408-420)             */
     RQ_OP_AND,          /* bitwise on 0/1                               (:446-455)             */
-    RQ_OP_OR,           /*                                              (:460-468)             */
+    RQ_OP_OR,           /*                                              (:460-468)
+                           An OR tree whose leaves all test one value for equality against constants
+                           (EQ, or only EQ_CHAR, or only EQ_VARCHAR; what `x IN (...)` parses to) is
+                           evaluated as one set-membership test, with no limit on its length.      */
     RQ_OP_LT, RQ_OP_LE, RQ_OP_GT, RQ_OP_GE,   /* signed compare -> 0/1  (:474-615)             */
     RQ_OP_EQ,           /* integer equality -> 0/1                      (:620-632)             */
     RQ_OP_NEQ,          /* 1 - EQ                                       (:1036-1043)           */

@@ -18,6 +18,7 @@
 #include <algorithm>
 #include <chrono>
 #include <functional>
+#include <tuple>
 
 #include "../../include/resql_b200.h"
 #include "rq_internal.h"
@@ -129,6 +130,8 @@ struct Options {
     bool graphs = true;                   // replayed plans are captured into CUDA graphs
     bool zone_skip = true;                // selections on sorted columns restrict the scan to a tile range
     int late_materialize = 1;             // 0 never, 1 where the early form cannot hold a materialize, 2 wherever it applies
+    int in_lists = 1;                     // OR trees of equality tests against constants as one set test (engine_exec.inl
+                                          // "IN lists"): 0 never, 1 lists of kInListMinInt / kInListMinStr values or more, 2 every list
     bool share_builds = true;             // sharded plans: replicated pure-scan builds are split over the ranks and all-reduced
     int64_t share_min_rows = 1 << 20;
     bool narrow = true;                   // host-buffer uploads send 8-byte columns over PCIe in the narrowest exact width
@@ -260,6 +263,7 @@ extern "C" int rq_set_option(const char* key, double value) {
     else if (k == "narrow") o.narrow = value != 0;
     else if (k == "zone_skip") o.zone_skip = value != 0;
     else if (k == "late_materialize") o.late_materialize = std::max(0, std::min((int)value, 2));
+    else if (k == "in_lists") o.in_lists = std::max(0, std::min((int)value, 2));
     else if (k == "share_builds") o.share_builds = value != 0;
     else if (k == "share_min_rows") o.share_min_rows = (int64_t)value;
     else if (k == "up_threads") o.up_threads = (int)value;
@@ -793,6 +797,9 @@ bool is_leaf(int op) { return op == RQ_OP_COL || op == RQ_OP_CONST || op == RQ_O
 // probe's matched entry (scan kernel variant LATE).
 constexpr int kOpRowId = 1000;
 constexpr int kPayloadEntry = -1;
+// Node only simplify_pipeline builds (never accepted from the ABI either): a = value, imm = key of a
+// constant set in g_inlists; 1 when the value is in the set (an IN list, engine_exec.inl "IN lists").
+constexpr int kOpInSet = 1001;
 bool is_binary(int op) {
     switch (op) {
         case RQ_OP_ADD: case RQ_OP_SUB: case RQ_OP_MUL: case RQ_OP_DIV: case RQ_OP_AND: case RQ_OP_OR:
@@ -842,7 +849,7 @@ struct HOpnd {           // host-level operand of a unit / value reference of a 
 };
 typedef HOpnd HRef;
 
-enum HOp : uint8_t { H_FCMP = 1, H_BIN = 2, H_MULI = 3, H_SEL = 4, H_PROBE = 5, H_FRANGE = 6 };
+enum HOp : uint8_t { H_FCMP = 1, H_BIN = 2, H_MULI = 3, H_SEL = 4, H_PROBE = 5, H_FRANGE = 6, H_INSET = 7 };
 
 // One unit of the host-level program (what tests/vm_model.py executes):
 //   H_FCMP  valid &= (x GOP imm)                      gop in D_LT..D_NE, x a column
@@ -851,6 +858,7 @@ enum HOp : uint8_t { H_FCMP = 1, H_BIN = 2, H_MULI = 3, H_SEL = 4, H_PROBE = 5, 
 //   H_SEL   t = (x & 0xff) ? y : z
 //   H_PROBE hash-join probe number aux
 //   H_FRANGE valid &= (imm <= x <= imm + imm2)         two H_FCMP on one column fused
+//   H_INSET t = (x in the constant set at device address imm)   (modelled by tests/vm_model_inset.py)
 // then  slot[dst] = t  if dst >= 0, and  valid &= (t & 0xff) != 0  if filt.
 struct HUnit {
     uint8_t op = 0, gop = 0;
@@ -983,6 +991,7 @@ struct Lowerer {
                 }
                 case RQ_OP_PAYLOAD: check_ref(i, nd.a); break;
                 case kOpRowId: break;
+                case kOpInSet: use(i, nd.a); break;
                 default:
                     if (is_binary(nd.op)) { use(i, nd.a); use(i, nd.b); }
                     else raise(RQ_ERR_INVALID, "node %d: unknown op %d", i, nd.op);
@@ -1105,6 +1114,7 @@ struct Lowerer {
                     break;
                 case RQ_OP_SELECT:
                     vlo[i] = std::min(vlo[nd.b], vlo[nd.c]); vhi[i] = std::max(vhi[nd.b], vhi[nd.c]); break;
+                case kOpInSet: vlo[i] = 0; vhi[i] = 1; break;
                 default: break;   // DIV, PROBE, PAYLOAD, strings: unknown
             }
         }

@@ -80,7 +80,8 @@ enum DOp : uint8_t {
     D_LD = 1, D_ADD, D_SUB, D_RSUB, D_MUL, D_DIV, D_RDIV, D_AND, D_OR,
     D_LT, D_LE, D_GT, D_GE, D_EQ, D_NE,
     D_EQC, D_EQV, D_NEC, D_NEV, D_LIKE, D_RLIKE,
-    D_SEL
+    D_SEL,
+    D_INSET         // U_GEN: t = (x in the constant set at imm), see InSetHeader
 };
 
 enum DSrc : uint8_t { S_NONE = 0, S_COL = 1, S_SLOT = 2, S_IMM = 3, S_STR = 4 };
@@ -139,6 +140,36 @@ struct UInsn {
     uint32_t zrel;      // byte offset of z; K_IMM: index   } yrel|zrel<<32 = span (unsigned)
 };
 static_assert(sizeof(UInsn) == 32, "UInsn must be 32 bytes");
+
+// ---- constant sets of IN lists (U_GEN D_INSET) -----------------------------------------------------
+// A set is one block of 64-bit words in device memory, built on the host (engine_exec.inl "IN lists"):
+// the header, then the data of its form.
+//   IS_BITMAP   integers: bit (x - a) of 32-bit words over [a, a + b]        one range test, one load
+//   IS_SORTED   integers: a sorted values                                    branchless binary search
+//   IS_CHAR     strings: open-addressing table of cap = a + 1 entries {hash, byte offset of the
+//   IS_VARCHAR  constant from the block start (0 = empty)}, then the NUL-terminated constants
+enum InSetForm : uint32_t { IS_BITMAP = 0, IS_SORTED = 1, IS_CHAR = 2, IS_VARCHAR = 3 };
+struct InSetHeader {
+    uint64_t form;
+    uint64_t a;          // IS_BITMAP: lowest value; IS_SORTED: count; IS_CHAR / IS_VARCHAR: table mask
+    uint64_t b;          // IS_BITMAP: highest value - lowest value
+    uint64_t pad;
+};
+static_assert(sizeof(InSetHeader) == 32, "the set data starts at word 4");
+
+// Hash of a string constant of a set and of a tuple's string: FNV-1a over the bytes in front of the
+// NUL; CHAR sets (`blank_pad`) leave out trailing blanks, which compareChar ignores.
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+inline uint64_t inset_str_hash(const char* s, bool blank_pad) {
+    int n = 0;
+    while (s[n] != '\0') n++;
+    if (blank_pad) while (n > 0 && s[n - 1] == ' ') n--;
+    uint64_t h = 0xcbf29ce484222325ULL;
+    for (int i = 0; i < n; i++) { h ^= (unsigned char)s[i]; h *= 0x100000001b3ULL; }
+    return h;
+}
 
 struct VRef {           // value reference used by sinks (keys, payloads, outputs)
     uint8_t  kind;      // UKind

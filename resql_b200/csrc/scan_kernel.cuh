@@ -230,6 +230,76 @@ __device__ __forceinline__ void reg_set(T (&a)[N], int i, T x) {
 }
 
 // ---- low-cardinality global group table (packed key) -----------------------------------------
+// The set test (U_GEN with D_INSET): which of the 8 tuples of a lane hold a value in the constant set S
+// (rq_internal.h InSetHeader), as a bit mask. The set is read through the read-only path; it is small
+// enough to stay in L2. Strings of tuples outside `valid` are not touched (they may lie past the column).
+// The operand is a staged column or a slot read in its width, or a string column (encode_program refuses
+// any other kind).
+// Not inlined, like str_like: inside the interpreter switch it would change the register allocation of
+// every kernel variant. It is an operation of the generic unit rather than a unit code of its own: a
+// case of its own in the unit switch changed the dispatch of every other unit, and Q3 took 4 % longer.
+// xa: shared address of the operand (staged column or slot); a string column is at sbase, sw bytes a row.
+__device__ __noinline__ uint32_t inset_unit(uint32_t xa, uint32_t xkind, const unsigned char* sbase, uint32_t sw, uint32_t tile,
+                                            int lane, const uint64_t* S, unsigned valid) {
+    int64_t v[kR];
+    if (xkind == K_STR) {
+#pragma unroll
+        for (int r = 0; r < kR; r++) v[r] = (int64_t)(sbase + ((size_t)tile * kTile + row_in_tile(r, lane)) * sw);
+    } else if (xkind == K_M64) {
+        ld_m64(xa + lane * 16, v);
+    } else if (xkind == K_M32) {
+        int32_t t[kR]; ld_m32(xa + lane * 8, t);
+#pragma unroll
+        for (int r = 0; r < kR; r++) v[r] = t[r];
+    } else {
+        uint32_t t[kR]; ld_m8(xa + lane * 2, t);
+#pragma unroll
+        for (int r = 0; r < kR; r++) v[r] = t[r];
+    }
+    const uint64_t form = __ldg(S), a = __ldg(S + 1), b = __ldg(S + 2);
+    uint32_t hit = 0;
+    if (form == IS_BITMAP) {
+        const uint32_t* bits = reinterpret_cast<const uint32_t*>(S + 4);
+#pragma unroll
+        for (int r = 0; r < kR; r++) {
+            const uint64_t d = (uint64_t)v[r] - a;
+            if (d <= b) hit |= ((__ldg(bits + (d >> 5)) >> (d & 31)) & 1u) << r;
+        }
+    } else if (form == IS_SORTED) {
+        // branchless binary search; the 8 searches of a lane advance together, so their loads are in
+        // flight at the same time
+        const int64_t* x = reinterpret_cast<const int64_t*>(S + 4);
+        uint32_t base[kR];
+#pragma unroll
+        for (int r = 0; r < kR; r++) base[r] = 0;
+        for (uint32_t len = (uint32_t)a; len > 1;) {
+            const uint32_t half = len >> 1;
+#pragma unroll
+            for (int r = 0; r < kR; r++) base[r] = __ldg(x + base[r] + half) <= v[r] ? base[r] + half : base[r];
+            len -= half;
+        }
+        if (a != 0) {
+#pragma unroll
+            for (int r = 0; r < kR; r++) hit |= (__ldg(x + base[r]) == v[r] ? 1u : 0u) << r;
+        }
+    } else {
+        const bool chr = form == IS_CHAR;
+        const char* blk = reinterpret_cast<const char*>(S);
+#pragma unroll 1
+        for (int r = 0; r < kR; r++) {
+            if (!((valid >> r) & 1)) continue;
+            const char* s = reinterpret_cast<const char*>(reg_at(v, r));
+            const uint64_t h = inset_str_hash(s, chr);
+            for (uint64_t i = h & a;; i = (i + 1) & a) {
+                const uint64_t off = __ldg(S + 4 + 2 * i + 1);
+                if (off == 0) break;
+                if (__ldg(S + 4 + 2 * i) == h && (chr ? str_eq_char(s, blk + off) : str_eq_varchar(s, blk + off))) { hit |= 1u << r; break; }
+            }
+        }
+    }
+    return hit;
+}
+
 __device__ __forceinline__ int group_table_slot(const KParams& P, uint64_t key) {
     uint64_t hh = mix64(key ^ 0x9E3779B97F4A7C15ULL);
     uint32_t i = (uint32_t)(hh & (kGroupTableCap - 1));
@@ -779,6 +849,14 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                                   in.zkind == K_IMM ? P.imm[in.zrel] : 0, e);
 #pragma unroll
                             for (int r = 0; r < kR; r++) t[r] = (t[r] & 0xff) ? b[r] : e[r];
+                            break;
+                        }
+                        case D_INSET: {   // x IN (constants): one membership test for the whole OR tree
+                            const bool str = in.xkind == K_STR;
+                            const uint32_t hit = inset_unit(xa, in.xkind, str ? P.str_ptr[in.xrel] : nullptr, str ? P.str_w[in.xrel] : 0,
+                                                            tile, lane, reinterpret_cast<const uint64_t*>(in.imm), valid);
+#pragma unroll
+                            for (int r = 0; r < kR; r++) t[r] = (hit >> r) & 1;
                             break;
                         }
                         default: break;   // D_LD: t = x

@@ -149,13 +149,18 @@ def debug_lower(plan, pipeline, impl, col_types, col_widths, col_min=None, col_m
     n = len(col_types)
     ty = (C.c_int32 * n)(*col_types)
     wi = (C.c_int32 * n)(*col_widths)
-    buf = C.create_string_buffer(1 << 16)
     mn = (C.c_int64 * n)(*col_min) if col_min is not None else None
     mx = (C.c_int64 * n)(*col_max) if col_max is not None else None
-    rc = lib.rq_debug_lower(C.byref(cplan), pipeline, impl, ty, wi, mn, mx, n, buf, len(buf))
-    if rc != 0:
-        raise EngineError(rc, lib.rq_last_error().decode())
-    return buf.value.decode()
+    size = 1 << 16
+    while True:       # (long IN lists print one line per set member)
+        buf = C.create_string_buffer(size)
+        rc = lib.rq_debug_lower(C.byref(cplan), pipeline, impl, ty, wi, mn, mx, n, buf, len(buf))
+        if rc == 0:
+            return buf.value.decode()
+        msg = lib.rq_last_error().decode()
+        if "buffer too small" not in msg or size >= 1 << 30:
+            raise EngineError(rc, msg)
+        size *= 4
 
 
 ABI_SYMBOLS = ["rq_init", "rq_shutdown", "rq_last_error", "rq_stream", "rq_set_option", "rq_dist_unique_id",
