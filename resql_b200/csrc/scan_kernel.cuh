@@ -1188,10 +1188,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                 // value goes into the accumulator of every group through the 0/1 group multiplier.
                 // sm_100a has no fused 64-bit multiply-add (IMAD.WIDE + IADD3 + IADD3.X), so the host
                 // picks the cheapest exact form per aggregate from the value bounds (upload
-                // statistics + interval arithmetic):
-                //   AM_P1   value < 2^24: one 32-bit accumulator, one IMAD per (group, tuple)
-                //   AM_P2   value < 2^48: two 32-bit accumulators for the low / high piece
+                // statistics + interval arithmetic; the first three need value >= 0):
+                //   AM_P1   value < 2^25: one 32-bit accumulator, one IMAD per (group, tuple)
                 //   AM_W64  value < 2^32: 64-bit accumulator, IMAD.WIDE.U32 + 64-bit add
+                //   AM_P2   value < 2^48: two 32-bit accumulators for the low / high piece
                 //   AM_FULL any int64   : 64-bit accumulator, wide multiply of the low word plus the
                 //                         high word's low product (wrap-around int64 sum)
                 // 32-bit accumulators are flushed to the global group table before they can wrap

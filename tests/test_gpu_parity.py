@@ -43,9 +43,9 @@ def test_fixture_matches_reference_engine(name, sf001, engine):
 
 
 @pytest.mark.parametrize("name", ["q1", "q6", "agg_linenumber", "agg_wrap", "agg_nogroup_minmax", "case_sum"])
-@pytest.mark.parametrize("rows", [0, 1, 1023, 1024, 1025, 5000, 300_001])
+@pytest.mark.parametrize("rows", [0, 1, 255, 256, 257, 1023, 1024, 1025, 5000, 300_001])
 def test_ragged_sizes_match_oracle(name, rows, engine):
-    """empty, single-row, tile-boundary and multi-CTA inputs (tile = 1024 tuples)"""
+    """empty, single-row, tile-boundary and multi-CTA inputs (tile = 256 tuples)"""
     d = load_plan_dict(name)
     data = tpch.generate(0.06, seed=1234, tables=("lineitem",))
     tabs = plan_tables(d, data)
