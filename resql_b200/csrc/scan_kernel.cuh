@@ -15,8 +15,10 @@
 // stage the guarded tail of a borrowed source, or the pairs of a cross source), prefetch_next (L2
 // prefetch of the next tile) and drain_ring (early exit on a full hash table). Repeated sink pieces
 // have one definition each: atomic_agg (hash aggregation and groupjoin), put_match (probe matches),
-// warp_group_slot (group-table slot of a flush), leader_key (a new dictionary key), reg_at / reg_set
-// (an element of a register array).
+// warp_group_slot (group-table slot of a flush), flush_groups (the groups a flush covers), leader_key
+// (a new dictionary key), reg_at / reg_set (an element of a register array). The materialize sink
+// (sink_emit) and the LOWAGG end flush (flush_lowagg) are functions; the program, the probe unit and
+// the other sinks are written in the kernel body (DESIGN §3.1).
 //
 // Aggregation (template parameter GR):
 //   GR = 1 / 4  register path: up to GR groups x kNAR aggregates live in registers for the whole
@@ -531,6 +533,60 @@ __device__ __forceinline__ void prefetch_next(const KParams& P, const Ring& g, u
     }
 }
 
+// ---- sink pieces ------------------------------------------------------------------------------
+// Kernel state changes only through reference parameters; NA / NK are the kernel's P.na / P.nk. The
+// other sinks stay in the kernel body: moved into functions, even verbatim, each changed the SASS of
+// the GR = 0 variants, and moving the probe unit that way cost Q3 8.5 % (profiles/r06_kernel_split_ab.txt).
+
+// Groups a flush covers (register path and LOWAGG): the warp's dictionary entries, or with no GROUP BY
+// key the one group if any lane aggregated a tuple.
+__device__ __forceinline__ int flush_groups(int NK, int ngroups, unsigned seen) {
+    int n = ngroups;
+    if (NK == 0) n = __any_sync(kFull, seen != 0) ? 1 : 0;
+    return n;
+}
+
+// Materialize (IMPL_EMIT): one atomic per warp tile, lanes take consecutive output ranges. `valid` is
+// read only.
+__device__ __forceinline__ void sink_emit(const KParams& P, const WarpCtx& c, unsigned valid) {
+    const int lane = c.lane;
+    const int cnt = __popc(valid);
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(kFull, incl, o);
+        if (lane >= o) incl += t;
+    }
+    const int total = __shfl_sync(kFull, incl, 31);
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(P.out_count, (unsigned long long)total);
+    base = __shfl_sync(kFull, base, 0);
+    int64_t pos = (int64_t)base + (incl - cnt);
+    // only the surviving tuples are visited (a selective pass leaves a few per warp tile)
+    for (unsigned todo = valid; todo; todo &= todo - 1) {
+        const int r = __ffs(todo) - 1;
+        if (pos < P.out_cap)
+            for (int k = 0; k < P.n_out; k++) P.out_col[k][pos] = ld_row(P, c, P.out[k], r);
+        pos++;
+    }
+}
+
+// End of the scan for IMPL_LOWAGG: warp-reduce the accumulators of the first n groups (at most P.G) and
+// add them to the global group table.
+template <int ND>
+__device__ __forceinline__ void flush_lowagg(const KParams& P, int lane, int NA, int NK, uint32_t sacc, int n,
+                                             const uint64_t (&dk)[ND]) {
+    if (n > P.G) n = P.G;
+    for (int e = 0; e < n; e++) {
+        const int slot = warp_group_slot(P, NK, reg_at(dk, e), lane);
+        for (int a = 0; a < NA; a++) {
+            const int kind = P.agg_kind[a];
+            const int64_t v = warp_reduce(lds_b64(sacc + ((e * NA + a) * 32 + lane) * 8), kind);
+            if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, v);
+        }
+    }
+}
+
 // LATE (instantiated with GR = 0 only): late materialization. The tile's row (pair) indices go to
 // the slot P.late_row_rel before the program runs, and a probe writes the reference of its matched
 // entry to slot P.late_ref_slot[p]; the materialize sink then writes these references as columns of
@@ -623,8 +679,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     // register path: warp-reduce every (group, aggregate) partial and add it to the global group table
     // (at the end of the scan, and every P.flush_tiles tiles so that 32-bit piece sums cannot wrap)
     auto flush_regs = [&]() {
-        int n = ngroups;
-        if (NK == 0) n = __any_sync(kFull, seen != 0) ? 1 : 0;
+        const int n = flush_groups(NK, ngroups, seen);
 #pragma unroll
         for (int g = 0; g < NG; g++) {
             if (g >= n) continue;
@@ -654,8 +709,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         return (uint64_t)lo + ((uint64_t)hi << 16);
     };
     auto flush_small = [&]() {
-        int n = ngroups;
-        if (NK == 0) n = __any_sync(kFull, seen != 0) ? 1 : 0;
+        const int n = flush_groups(NK, ngroups, seen);
 #pragma unroll
         for (int g = 0; g < NG; g++) {
             if (g >= n) continue;
@@ -1474,26 +1528,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     }
                 }
             } else if (sink == IMPL_EMIT) {
-                // one atomic per warp tile: lanes take consecutive output ranges
-                const int cnt = __popc(valid);
-                int incl = cnt;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int t = __shfl_up_sync(kFull, incl, o);
-                    if (lane >= o) incl += t;
-                }
-                const int total = __shfl_sync(kFull, incl, 31);
-                unsigned long long base = 0;
-                if (lane == 0) base = atomicAdd(P.out_count, (unsigned long long)total);
-                base = __shfl_sync(kFull, base, 0);
-                int64_t pos = (int64_t)base + (incl - cnt);
-                // only the surviving tuples are visited (a selective pass leaves a few per warp tile)
-                for (unsigned todo = valid; todo; todo &= todo - 1) {
-                    const int r = __ffs(todo) - 1;
-                    if (pos < P.out_cap)
-                        for (int k = 0; k < P.n_out; k++) P.out_col[k][pos] = ld_row(P, c, P.out[k], r);
-                    pos++;
-                }
+                sink_emit(P, c, valid);
             }
         }
 
@@ -1527,21 +1562,9 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     // ---- flush the per-warp accumulators of the low-cardinality aggregate -------------------
     if (GR > 0 || sink == IMPL_LOWAGG) {
         __syncwarp();
-        int n = ngroups;
-        if (NK == 0) n = __any_sync(kFull, seen != 0) ? 1 : 0;
-        if (GR > 0) {
-            flush_regs();
-        } else {
-            if (n > P.G) n = P.G;
-            for (int e = 0; e < n; e++) {
-                const int slot = warp_group_slot(P, NK, reg_at(dk, e), lane);
-                for (int a = 0; a < NA; a++) {
-                    const int kind = P.agg_kind[a];
-                    const int64_t v = warp_reduce(lds_b64(sacc + ((e * NA + a) * 32 + lane) * 8), kind);
-                    if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, v);
-                }
-            }
-        }
+        const int n = flush_groups(NK, ngroups, seen);
+        if (GR > 0) flush_regs();
+        else flush_lowagg(P, lane, NA, NK, sacc, n, dk);
     }
 }
 
