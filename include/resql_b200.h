@@ -79,7 +79,10 @@ void* rq_stream(void);
  * references and gather their columns afterwards, up to 64 columns; 2: that form wherever it applies),
  * "in_lists" (OR trees of equality tests of one value against constants as one set test: 0 never, keeping
  * one compare per value; 1 = default: integer lists of 2 values or more, string lists of 4 or more;
- * 2: every list of 2 values or more).
+ * 2: every list of 2 values or more),
+ * "sink_rounds" (materialize pipelines whose computed outputs need more than 12 live values store them in
+ * rounds that each fit, up to 64 outputs: 0 never; 1 = default: only where the single sink cannot hold
+ * the values; 2: wherever it applies).
  * Defaults are the production choices; the parity tests force rarely taken paths. */
 int rq_set_option(const char* key, double value);
 

@@ -130,6 +130,8 @@ struct Options {
     bool graphs = true;                   // replayed plans are captured into CUDA graphs
     bool zone_skip = true;                // selections on sorted columns restrict the scan to a tile range
     int late_materialize = 1;             // 0 never, 1 where the early form cannot hold a materialize, 2 wherever it applies
+    int sink_rounds = 1;                  // materialize values in rounds (engine_exec.inl "sink rounds"): 0 never, 1 where
+                                          // the single sink cannot hold the values, 2 wherever it applies
     int in_lists = 1;                     // OR trees of equality tests against constants as one set test (engine_exec.inl
                                           // "IN lists"): 0 never, 1 lists of kInListMinInt / kInListMinStr values or more, 2 every list
     bool share_builds = true;             // sharded plans: replicated pure-scan builds are split over the ranks and all-reduced
@@ -210,7 +212,8 @@ extern "C" int rq_init(int device) {
         for (int gr : {0, 1, 4})
             for (bool cross : {false, true})
                 for (bool late : {false, true})
-                    CK(cudaFuncSetAttribute(scan_kernel_for(gr, cross, late), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+                    for (bool rounds : {false, true})
+                        CK(cudaFuncSetAttribute(scan_kernel_for(gr, cross, late, rounds), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         E.init = true;
         return RQ_OK;
     } catch (RqError& e) {
@@ -263,6 +266,7 @@ extern "C" int rq_set_option(const char* key, double value) {
     else if (k == "narrow") o.narrow = value != 0;
     else if (k == "zone_skip") o.zone_skip = value != 0;
     else if (k == "late_materialize") o.late_materialize = std::max(0, std::min((int)value, 2));
+    else if (k == "sink_rounds") o.sink_rounds = std::max(0, std::min((int)value, 2));
     else if (k == "in_lists") o.in_lists = std::max(0, std::min((int)value, 2));
     else if (k == "share_builds") o.share_builds = value != 0;
     else if (k == "share_min_rows") o.share_min_rows = (int64_t)value;
@@ -868,6 +872,7 @@ struct HUnit {
     bool filt = false;
     int aux = 0;
     bool n32 = false;        // both multiplication factors proven to lie in [0, 2^32)
+    int round = 0;           // sink rounds: 0 the prefix, k + 1 round k
 };
 
 struct Lowerer {
@@ -885,6 +890,12 @@ struct Lowerer {
     HRef hprobe_key[kMaxProbes][kMaxKeys];
     int n_slots = 0;
     int row_slot = -1;                // slot of the kOpRowId node (late materialization)
+    // sink rounds (engine_exec.inl "sink rounds"): round k stores values [round_val_end[k - 1],
+    // round_val_end[k]); empty: one sink after the whole program
+    std::vector<int> round_val_end;
+    int cur_round = 0;                // the round of the units emitted now
+    bool out_of_slots = false;        // the lowering failed for want of a value slot
+    bool allow_rounds = true;         // the pipeline may take the round form
 
     std::vector<int> uses;            // consumers per node
     std::vector<int> last_use;        // last consuming node index (n = sink)
@@ -909,6 +920,7 @@ struct Lowerer {
         if ((int)prog.size() >= kMaxInsn) raise(RQ_ERR_UNSUPPORTED, "program longer than %d units", kMaxInsn);
         HUnit u;
         u.op = op; u.gop = gop;
+        u.round = cur_round;
         prog.push_back(u);
         return prog.back();
     }
@@ -938,12 +950,23 @@ struct Lowerer {
 
     int alloc_slot() {
         if (!free_slots.empty()) { int s = free_slots.back(); free_slots.pop_back(); return s; }
+        if (n_slots >= kMaxSlots) out_of_slots = true;
         if (n_slots >= kMaxSlots) raise(RQ_ERR_UNSUPPORTED, "expression needs more than %d live temporaries", kMaxSlots);
         return n_slots++;
     }
     void release_dead(int at) {   // free slots of nodes whose last use is `at`
         for (int i = 0; i < n; i++)
             if (slot[i] >= 0 && last_use[i] == at) { free_slots.push_back(slot[i]); slot[i] = -2 - slot[i]; }
+    }
+
+    // back to the state before prepare(), keeping round_val_end (a second lowering of the pipeline)
+    void reset() {
+        prog.clear(); hkey.clear(); hout.clear();
+        for (HRef& h : hagg_src) h = HRef();
+        for (auto& k : hprobe_key) for (HRef& h : k) h = HRef();
+        n_slots = 0; row_slot = -1; cur_round = 0; out_of_slots = false;
+        free_slots.clear();
+        n_imm = 0;
     }
 
     void prepare() {

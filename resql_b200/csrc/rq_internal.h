@@ -331,6 +331,17 @@ struct KParams {
     uint32_t       late_row_rel;
     uint8_t        late_ref_slot[kMaxProbes];
     int32_t        late;                 // launch the LATE variant
+    // sink rounds (kernel variant ROUNDS, materialize only; engine_exec.inl "sink rounds"): units
+    // [0, prefix_end) are the prefix, which holds every filter and probe; after it the tile's output
+    // positions are located once. Round k then runs units [round_unit_end[k - 1], round_unit_end[k])
+    // (the first round starts at prefix_end) and stores values [round_val_end[k - 1], round_val_end[k])
+    // into their output columns. (Behind every other field, like the cross and late fields.)
+    int32_t        n_rounds;             // 0: the pipeline has the single sink of the other variants
+    int32_t        prefix_end;
+    uint16_t       round_unit_end[kMaxLateOut];
+    uint8_t        round_val_end[kMaxLateOut];
+    VRef           rval[kMaxLateOut];    // the sink values, in value (= output column) order
+    int64_t*       rout_col[kMaxLateOut];
 };
 
 }  // namespace rq

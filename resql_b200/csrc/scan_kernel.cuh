@@ -17,8 +17,9 @@
 // have one definition each: atomic_agg (hash aggregation and groupjoin), put_match (probe matches),
 // warp_group_slot (group-table slot of a flush), flush_groups (the groups a flush covers), leader_key
 // (a new dictionary key), reg_at / reg_set (an element of a register array). The materialize sink
-// (sink_emit) and the LOWAGG end flush (flush_lowagg) are functions; the program, the probe unit and
-// the other sinks are written in the kernel body (DESIGN §3.1).
+// (sink_emit, made of emit_locate and the stores) and the LOWAGG end flush (flush_lowagg) are functions;
+// the program, the probe unit and the other sinks are written in the kernel body (DESIGN §3.1). The
+// round variant (ROUNDS) runs the program in pieces around emit_locate and emit_put.
 //
 // Aggregation (template parameter GR):
 //   GR = 1 / 4  register path: up to GR groups x kNAR aggregates live in registers for the whole
@@ -546,10 +547,9 @@ __device__ __forceinline__ int flush_groups(int NK, int ngroups, unsigned seen) 
     return n;
 }
 
-// Materialize (IMPL_EMIT): one atomic per warp tile, lanes take consecutive output ranges. `valid` is
-// read only.
-__device__ __forceinline__ void sink_emit(const KParams& P, const WarpCtx& c, unsigned valid) {
-    const int lane = c.lane;
+// Materialize (IMPL_EMIT): the output position of the lane's first surviving tuple. One atomic per warp
+// tile, lanes take consecutive output ranges.
+__device__ __forceinline__ int64_t emit_locate(const KParams& P, int lane, unsigned valid) {
     const int cnt = __popc(valid);
     int incl = cnt;
 #pragma unroll
@@ -561,12 +561,28 @@ __device__ __forceinline__ void sink_emit(const KParams& P, const WarpCtx& c, un
     unsigned long long base = 0;
     if (lane == 0) base = atomicAdd(P.out_count, (unsigned long long)total);
     base = __shfl_sync(kFull, base, 0);
-    int64_t pos = (int64_t)base + (incl - cnt);
+    return (int64_t)base + (incl - cnt);
+}
+
+// Materialize (IMPL_EMIT). `valid` is read only.
+__device__ __forceinline__ void sink_emit(const KParams& P, const WarpCtx& c, unsigned valid) {
+    int64_t pos = emit_locate(P, c.lane, valid);
     // only the surviving tuples are visited (a selective pass leaves a few per warp tile)
     for (unsigned todo = valid; todo; todo &= todo - 1) {
         const int r = __ffs(todo) - 1;
         if (pos < P.out_cap)
             for (int k = 0; k < P.n_out; k++) P.out_col[k][pos] = ld_row(P, c, P.out[k], r);
+        pos++;
+    }
+}
+
+// One round of the round form (ROUNDS): the sink values [v0, v1) of the surviving tuples go to their
+// output columns from `pos`, the position emit_locate found for the lane before the first round.
+__device__ __forceinline__ void emit_put(const KParams& P, const WarpCtx& c, unsigned valid, int64_t pos, int v0, int v1) {
+    for (unsigned todo = valid; todo; todo &= todo - 1) {
+        const int r = __ffs(todo) - 1;
+        if (pos < P.out_cap)
+            for (int k = v0; k < v1; k++) P.rout_col[k][pos] = ld_row(P, c, P.rval[k], r);
         pos++;
     }
 }
@@ -591,11 +607,15 @@ __device__ __forceinline__ void flush_lowagg(const KParams& P, int lane, int NA,
 // the slot P.late_row_rel before the program runs, and a probe writes the reference of its matched
 // entry to slot P.late_ref_slot[p]; the materialize sink then writes these references as columns of
 // a record that rq_late_gather resolves into values.
-template <int GR, bool CROSS = false, bool LATE = false>
+// ROUNDS (instantiated with GR = 0 and LATE only): sink rounds of a materialize (KParams::n_rounds). Per
+// tile the prefix units run, the output positions are located once, then every round runs its units and
+// stores its values, so the value slots bound one round instead of the whole sink.
+template <int GR, bool CROSS = false, bool LATE = false, bool ROUNDS = false>
 __global__ void __launch_bounds__(kMaxWarps * 32, 1)
 rq_scan_kernel(const __grid_constant__ KParams P) {
     static_assert(!CROSS || GR == 0, "the cross-source variant has the generic sinks only");
     static_assert(!LATE || GR == 0, "the late variant has the generic sinks only");
+    static_assert(!ROUNDS || (GR == 0 && !CROSS && LATE), "the round variant is the late one with rounds");
     constexpr int NG = GR > 0 ? GR : 1;                 // register groups
     constexpr int ND = GR > 0 ? GR : kLowCardMaxGroups; // dictionary entries
     // lane / warp-region base are used everywhere; they are made opaque so that the compiler keeps
@@ -784,9 +804,13 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             }
         }
 
-        // ---- 1. the program ---------------------------------------------------------------
-        const int n_insn = P.n_insn;
-        for (int pc = 0; pc < n_insn; pc++) {
+        // ---- 1. the program (ROUNDS: the prefix, then the units of each round after the locate
+        //         or the previous round's stores) --------------------------------------------
+        int64_t rpos = 0;
+        int pc0 = 0;
+        for (int rd = -1;; rd++) {     // the parts of the program: units [pc0, n_insn) of part rd
+        const int n_insn = !ROUNDS ? P.n_insn : rd < 0 ? P.prefix_end : (int)P.round_unit_end[rd];
+        for (int pc = pc0; pc < n_insn; pc++) {
             const uint4 w0 = lds_v4b32(prog + pc * 32), w1 = lds_v4b32(prog + pc * 32 + 16);
             UInsn in;
             in.code = (uint8_t)w0.x; in.flags = (uint8_t)(w0.x >> 8); in.gop = (uint8_t)(w0.x >> 16); in.aux = (uint8_t)(w0.x >> 24);
@@ -1152,9 +1176,26 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             }
 #undef RQ_FINISH
         }
+        // End of one part of the program. The other variants run the whole program as one part. ROUNDS:
+        // the prefix (rd = -1) is followed by the locate and round rd by its stores, then the units of
+        // round rd + 1 run. No unit after the prefix drops a tuple, so the positions located once hold
+        // for every round.
+        if constexpr (ROUNDS) {
+            if (rd < 0) {
+                if (!__any_sync(kFull, valid != 0)) break;      // every tuple dropped: no round runs
+                rpos = emit_locate(P, lane, valid);
+            } else {
+                emit_put(P, c, valid, rpos, rd == 0 ? 0 : P.round_val_end[rd - 1], P.round_val_end[rd]);
+            }
+            if (rd + 1 == P.n_rounds) break;                    // the last round stored its values
+            pc0 = n_insn;                                       // round rd + 1 starts where this part ended
+        } else {
+            break;
+        }
+        }   // (the parts of the program; the loop body above is not indented for them)
 
         // ---- 2. the sink --------------------------------------------------------------------
-        if (__any_sync(kFull, valid != 0)) {
+        if (!ROUNDS && __any_sync(kFull, valid != 0)) {
             if (GR > 0) {
                 // register path: group match -> 0/1 multipliers -> accumulate
                 uint32_t m[NG][kR];
@@ -1569,9 +1610,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 }
 
 // The instantiations of the scan kernel and the one a launch uses: gr is the number of register
-// groups (0, 1 or 4); the cross-source and late variants exist for gr = 0 only and take precedence.
+// groups (0, 1 or 4); the cross-source, late and round variants exist for gr = 0 only and take precedence.
 using ScanKernel = void (*)(KParams);
-inline ScanKernel scan_kernel_for(int gr, bool cross, bool late) {
+inline ScanKernel scan_kernel_for(int gr, bool cross, bool late, bool rounds) {
+    if (rounds) return rq_scan_kernel<0, false, true, true>;
     if (late) return cross ? rq_scan_kernel<0, true, true> : rq_scan_kernel<0, false, true>;
     if (cross) return rq_scan_kernel<0, true>;
     return gr == 4 ? rq_scan_kernel<4> : gr == 1 ? rq_scan_kernel<1> : rq_scan_kernel<0>;
