@@ -12,6 +12,7 @@ namespace rq {
 // rq_init), so that per-query hash tables and intermediates are recycled instead of going
 // through cudaMalloc / cudaFree every time
 // ------------------------------------------------------------------------------------------
+#ifndef __CUDACC_RTC__     // (host code: not part of a run-time compiled specialization, jit.h)
 inline cudaStream_t& alloc_stream() { static cudaStream_t s = nullptr; return s; }
 template <typename T>
 inline cudaError_t dmalloc(T** p, size_t bytes) {
@@ -20,6 +21,7 @@ inline cudaError_t dmalloc(T** p, size_t bytes) {
 inline void dfree(void* p) {
     if (p) cudaFreeAsync(p, alloc_stream());
 }
+#endif
 
 // ------------------------------------------------------------------------------------------
 // PTX helpers: mbarrier + TMA bulk copy

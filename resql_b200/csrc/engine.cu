@@ -28,6 +28,7 @@
 #include "exchange_kernels.cuh"
 #include "dist.h"
 #include "host_narrow.h"
+#include "jit.h"
 #include <thread>
 #include <atomic>
 #include <mutex>
@@ -140,6 +141,7 @@ struct Options {
     int up_threads = 0;                   // host-buffer uploads: converting threads (0 = all cores of this rank's share)
     int up_chunk_krows = 512;             //                      rows per conversion / DMA chunk, in 1024 rows
     bool trace = false;                   // per-step wall-clock trace on stderr
+    bool specialize = true;               // scan launches run a kernel compiled for their pipeline (jit.h)
 };
 
 struct Engine {
@@ -273,6 +275,7 @@ extern "C" int rq_set_option(const char* key, double value) {
     else if (k == "up_threads") o.up_threads = (int)value;
     else if (k == "up_chunk_krows") o.up_chunk_krows = std::max(1, std::min((int)value, 8192));
     else if (k == "trace") o.trace = value != 0;
+    else if (k == "specialize") o.specialize = value != 0;
     else return fail(RQ_ERR_INVALID, "rq_set_option: unknown option '%s'", key);
     return RQ_OK;
 }

@@ -10,6 +10,7 @@
 
 namespace rq {
 
+#ifndef __CUDACC_RTC__     // (host code: not part of a run-time compiled specialization, jit.h)
 struct HashTableDev {
     DHashTable d{};
     uint64_t capacity = 0;
@@ -18,6 +19,7 @@ struct HashTableDev {
         dfree(d.ent); dfree(d.bloom); dfree(d.dbits); dfree(d.darr);
     }
 };
+#endif
 
 constexpr uint64_t kTagLocked = 1ULL;
 // A full table is detected by its LOAD (entries are counted per warp tile against DHashTable::limit,

@@ -53,6 +53,7 @@ struct FlagBlock {
     uint64_t reserved;
     uint64_t popcount;      // shared build: set bits of the all-reduced bitmap
 };
+#ifndef __CUDACC_RTC__     // (NVRTC has no offsetof: a run-time compiled kernel, jit.h, gets the one word index it uses below)
 static_assert(offsetof(FlagBlock, overflow) == 0, "FlagBlock layout");
 static_assert(offsetof(FlagBlock, ht_full) == 4, "FlagBlock layout");
 static_assert(offsetof(FlagBlock, err) == 8, "FlagBlock layout");
@@ -74,6 +75,10 @@ constexpr int kFlagWordEntries  = offsetof(FlagBlock, entries) / 4;
 constexpr int kFlagWordPopcount = offsetof(FlagBlock, popcount) / 4;
 // KParams::ht_full points at FlagBlock::ht_full; the direct-address build raises dup_key through it
 constexpr int kDupKeyFromHtFull = (offsetof(FlagBlock, dup_key) - offsetof(FlagBlock, ht_full)) / 4;
+static_assert(kDupKeyFromHtFull == 2, "the NVRTC value below");
+#else
+constexpr int kDupKeyFromHtFull = 2;
+#endif
 
 // ---- operation codes shared by the host-level program and the device encoding ----------------
 enum DOp : uint8_t {

@@ -114,6 +114,60 @@ struct WarpCtx {
     int      lane;
 };
 
+// ---- what the host knows at launch ------------------------------------------------------------
+// The kernel reads every field that stays the same across executions of a pipeline on the same
+// tables (program encoding, operand kinds and offsets, sink descriptors, stage layout, probe flags)
+// through a spec type. GenericSpec reads them from KParams at run time; that is what the
+// ahead-of-time kernels use. A specialization compiled at run time (jit.h) provides the same
+// accessors as constants, so the unit switch, the operand-kind dispatch and the sink's form branches
+// fold away. Pointers, row counts, tile ranges, capacities and immediates are always read from KParams.
+// The baked fields: F(type, accessor, value) for a scalar, A(type, accessor, length, value of element i)
+// for an array, PR / PR2 the same per probe p (jit.h generates a specialization from this list).
+#define RQ_SPEC_FIELDS(F, A, PR, PR2)                                                                         \
+    F(int, n_insn, P.n_insn) F(int, sink, P.sink) F(int, na, P.na) F(int, nk, P.nk) F(int, key32, P.key32)    \
+    F(int, G, P.G) F(int, expand_probe, P.expand_probe) F(int, n_out, P.n_out)                               \
+    F(int, n_cols, P.n_cols) F(int, n_runs, P.n_runs) F(int, stages, P.stages)                               \
+    F(uint32_t, stage_bytes, P.stage_bytes) F(uint32_t, warp_off, P.warp_off) F(uint32_t, warp_bytes, P.warp_bytes) \
+    F(uint32_t, slots_rel, P.slots_rel) F(uint32_t, acc_rel, P.acc_rel) F(uint32_t, prog_off, P.prog_off)     \
+    F(int, l2_prefetch, P.l2_prefetch) F(int, stream_hint, P.stream_hint)                                    \
+    F(uint32_t, ht_direct, P.ht.direct) F(uint32_t, ht_packed, P.ht.packed) F(int, ht_nk, P.ht.nk)            \
+    A(int, ht_key_kind, kMaxKeys, P.ht.key_kind[i])                                                          \
+    A(VRef, key, kMaxKeys, P.key[i]) A(int, key_shift, kMaxKeys, P.key_shift[i]) A(int, key_bits, kMaxKeys, P.key_bits[i]) \
+    A(int, agg_kind, kMaxAggs, P.agg_kind[i]) A(int, agg_mode, kMaxAggs, P.agg_mode[i])                      \
+    A(int, agg_shift, kMaxAggs, P.agg_shift[i]) A(uint32_t, agg_desc, kMaxAggs, P.agg_desc[i])                \
+    A(VRef, agg_src, kMaxAggs, P.agg_src[i]) A(VRef, out, kMaxOut, P.out[i])                                  \
+    A(uint32_t, run_off, kMaxStagedCols, P.run_off[i]) A(uint32_t, run_bytes, kMaxStagedCols, P.run_bytes[i])  \
+    A(uint32_t, run_stride, kMaxStagedCols, P.run_stride[i])                                                 \
+    A(uint32_t, col_off, kMaxStagedCols, P.col_off[i]) A(int, col_w, kMaxStagedCols, P.col_w[i])              \
+    PR(int, pr_fetch, pr.fetch) PR(uint32_t, pr_direct, pr.ht.direct)                         \
+    PR(int, pr_bloom_only, pr.bloom_only) PR(int, pr_single, pr.single)                       \
+    PR(int, pr_n_out, pr.n_out) PR(int, pr_nk, pr.ht.nk) PR(bool, pr_bloom, pr.ht.bloom != nullptr) \
+    PR2(int, pr_key_kind, kMaxKeys, pr.ht.key_kind[i]) PR2(VRef, pr_key, kMaxKeys, pr.key[i]) \
+    PR2(int, pr_out_slot, kMaxOut, pr.out_slot[i]) PR2(int, pr_pay_word, kMaxOut, pr.pay_word[i])
+struct GenericSpec {
+    static constexpr bool kFixed = false;
+    // unit pc of the program, from its copy in shared memory at `prog`
+    static __device__ __forceinline__ UInsn insn(const KParams&, uint32_t prog, int pc) {
+        const uint4 w0 = lds_v4b32(prog + pc * 32), w1 = lds_v4b32(prog + pc * 32 + 16);
+        UInsn in;
+        in.code = (uint8_t)w0.x; in.flags = (uint8_t)(w0.x >> 8); in.gop = (uint8_t)(w0.x >> 16); in.aux = (uint8_t)(w0.x >> 24);
+        in.xkind = (uint8_t)w0.y; in.ykind = (uint8_t)(w0.y >> 8); in.zkind = (uint8_t)(w0.y >> 16);
+        in.xrel = w0.z; in.dstrel = w0.w;
+        in.imm = (int64_t)((uint64_t)w1.x | ((uint64_t)w1.y << 32));
+        in.yrel = w1.z; in.zrel = w1.w;
+        return in;
+    }
+#define RQ_SPEC_FIELD(T, NAME, EXPR) static __device__ __forceinline__ T NAME(const KParams& P) { return EXPR; }
+#define RQ_SPEC_ARRAY(T, NAME, N, EXPR) static __device__ __forceinline__ T NAME(const KParams& P, int i) { return EXPR; }
+#define RQ_SPEC_PROBE(T, NAME, EXPR) static __device__ __forceinline__ T NAME(const DProbe& pr, int) { return EXPR; }
+#define RQ_SPEC_PROBE2(T, NAME, N, EXPR) static __device__ __forceinline__ T NAME(const DProbe& pr, int, int i) { return EXPR; }
+    RQ_SPEC_FIELDS(RQ_SPEC_FIELD, RQ_SPEC_ARRAY, RQ_SPEC_PROBE, RQ_SPEC_PROBE2)
+#undef RQ_SPEC_FIELD
+#undef RQ_SPEC_ARRAY
+#undef RQ_SPEC_PROBE
+#undef RQ_SPEC_PROBE2
+};
+
 // any operand kind -> 8 int64 values (rare forms, group keys, aggregate inputs)
 __device__ __forceinline__ void fetch(const KParams& P, const WarpCtx& c, int kind, bool slot,
                                       uint32_t off, int64_t imm, int64_t (&v)[kR]) {
@@ -171,12 +225,13 @@ __device__ __forceinline__ int64_t ld_row(const KParams& P, const WarpCtx& c, VR
 // packed group key: every key is a bit field of one word. In the 32-bit form (P.key32) every
 // field is wide enough for its value by construction (pack_group_key sizes it from the value bounds
 // or the physical width), so no masking is needed.
+template <class Sp>
 __device__ __forceinline__ void pack_keys32(const KParams& P, const WarpCtx& c, uint32_t (&k32)[kR]) {
 #pragma unroll
     for (int r = 0; r < kR; r++) k32[r] = 0;
-    for (int j = 0; j < P.nk; j++) {
-        const VRef vr = P.key[j];
-        const int sh = P.key_shift[j];
+    for (int j = 0; j < Sp::nk(P); j++) {
+        const VRef vr = Sp::key(P, j);
+        const int sh = Sp::key_shift(P, j);
         const uint32_t base = ((vr.slot & 1) ? c.wbase : c.stage) + ((uint32_t)vr.off16 << 4);
         if (vr.kind == K_M8) {
             uint32_t t[kR];
@@ -197,21 +252,22 @@ __device__ __forceinline__ void pack_keys32(const KParams& P, const WarpCtx& c, 
         }
     }
 }
+template <class Sp>
 __device__ __forceinline__ void pack_keys(const KParams& P, const WarpCtx& c, uint64_t (&key)[kR]) {
-    if (P.key32) {
+    if (Sp::key32(P)) {
         uint32_t k32[kR];
-        pack_keys32(P, c, k32);
+        pack_keys32<Sp>(P, c, k32);
 #pragma unroll
         for (int r = 0; r < kR; r++) key[r] = k32[r];
         return;
     }
 #pragma unroll
     for (int r = 0; r < kR; r++) key[r] = 0;
-    for (int j = 0; j < P.nk; j++) {
+    for (int j = 0; j < Sp::nk(P); j++) {
         int64_t kv[kR];
-        fetch_vref(P, c, P.key[j], kv);
-        const int sh = P.key_shift[j];
-        const uint64_t mask = P.key_bits[j] >= 64 ? ~0ULL : ((1ULL << P.key_bits[j]) - 1);
+        fetch_vref(P, c, Sp::key(P, j), kv);
+        const int sh = Sp::key_shift(P, j);
+        const uint64_t mask = Sp::key_bits(P, j) >= 64 ? ~0ULL : ((1ULL << Sp::key_bits(P, j)) - 1);
 #pragma unroll
         for (int r = 0; r < kR; r++) key[r] |= ((uint64_t)kv[r] & mask) << sh;
     }
@@ -351,10 +407,11 @@ __device__ __forceinline__ void group_table_add(const KParams& P, int slot, int 
 }
 
 // adds tuple r to aggregate a, whose word is acc[a] (hash aggregation and groupjoin entries)
+template <class Sp>
 __device__ __forceinline__ void atomic_agg(const KParams& P, const WarpCtx& c, uint64_t* acc, int a, int r) {
-    const int kind = P.agg_kind[a];
+    const int kind = Sp::agg_kind(P, a);
     if (kind == RQ_AGG_COUNT) { atomicAdd((unsigned long long*)&acc[a], 1ULL); return; }
-    const int64_t v = ld_row(P, c, P.agg_src[a], r);
+    const int64_t v = ld_row(P, c, Sp::agg_src(P, a), r);
     if (kind == RQ_AGG_SUM) atomicAdd((unsigned long long*)&acc[a], (unsigned long long)v);
     else if (kind == RQ_AGG_MIN) atomicMin((long long*)&acc[a], (long long)v);
     else atomicMax((long long*)&acc[a], (long long)v);
@@ -371,12 +428,12 @@ __device__ __forceinline__ uint64_t leader_key(unsigned unk, const uint64_t (&ke
 
 // a probe match of the tuple at `row`: the entry's payload words go to their value slots and, in the
 // late variant, the entry reference `ref` to the probe's reference slot
-template <bool LATE>
+template <bool LATE, class Sp>
 __device__ __forceinline__ void put_match(const KParams& P, const DProbe& pr, int p, uint32_t wbase, int row,
                                           const uint64_t* ent, int64_t ref) {
-    for (int q = 0; q < pr.n_out; q++)
-        if (pr.out_slot[q] != 0xff)
-            sts_b64(wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8) + row * 8, (int64_t)ent[pr.pay_word[q]]);
+    for (int q = 0; q < Sp::pr_n_out(pr, p); q++)
+        if (Sp::pr_out_slot(pr, p, q) != 0xff)
+            sts_b64(wbase + Sp::slots_rel(P) + Sp::pr_out_slot(pr, p, q) * (kTile * 8) + row * 8, (int64_t)ent[Sp::pr_pay_word(pr, p, q)]);
     if constexpr (LATE) {
         if (P.late_ref_slot[p] != 0xff)
             sts_b64(wbase + P.slots_rel + P.late_ref_slot[p] * (kTile * 8) + row * 8, ref);
@@ -468,19 +525,20 @@ struct Ring {
 
 // One lane issues the bulk copies of all staged columns of a tile into stage s (uniform operands)
 // after arming the stage's barrier with its byte count. The guarded tile is staged by plain loads.
+template <class Sp>
 __device__ __forceinline__ void issue_tile(const KParams& P, const Ring& g, uint32_t tile, int s) {
     if (tile == g.guarded_tile) return;
     if (elect_one()) {
         const uint32_t bar = g.bars + s * 8;
-        const uint32_t dst0 = g.wbase + s * P.stage_bytes;
+        const uint32_t dst0 = g.wbase + s * Sp::stage_bytes(P);
         const uint32_t t32 = tile;
-        mbar_expect_tx_s(bar, P.stage_bytes);
+        mbar_expect_tx_s(bar, Sp::stage_bytes(P));
         if (g.hint) {
             for (int c = 0; c < g.n_runs; c++)
-                tma_bulk_g2s_hint(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar, g.policy);
+                tma_bulk_g2s_hint(dst0 + Sp::run_off(P, c), P.run_ptr[c] + (size_t)t32 * Sp::run_stride(P, c), Sp::run_bytes(P, c), bar, g.policy);
         } else {
             for (int c = 0; c < g.n_runs; c++)
-                tma_bulk_g2s_s(dst0 + P.run_off[c], P.run_ptr[c] + (size_t)t32 * P.run_stride[c], P.run_bytes[c], bar);
+                tma_bulk_g2s_s(dst0 + Sp::run_off(P, c), P.run_ptr[c] + (size_t)t32 * Sp::run_stride(P, c), Sp::run_bytes(P, c), bar);
         }
     }
 }
@@ -501,7 +559,7 @@ __device__ __forceinline__ void drain_ring(const Ring& g, uint32_t tile, int s, 
 // The tile at c.row0 is in stage s after this: the bulk copies have landed, or the guarded tail of
 // a borrowed source was staged with plain loads (zeros past n_rows), or the warp staged the pairs of
 // a cross source itself.
-template <bool CROSS>
+template <bool CROSS, class Sp>
 __device__ __forceinline__ void stage_tile(const KParams& P, const WarpCtx& c, const Ring& g, uint32_t tile, int s,
                                            uint32_t phase, int64_t n_rows, uint64_t n_inner, int n_cols) {
     if constexpr (CROSS) {
@@ -509,11 +567,11 @@ __device__ __forceinline__ void stage_tile(const KParams& P, const WarpCtx& c, c
     } else if (n_cols > 0) {
         if (tile == g.guarded_tile) {
             const int64_t rows = n_rows - c.row0;
-            for (int col = 0; col < P.n_cols; col++) {
-                const int w = P.col_w[col];
+            for (int col = 0; col < Sp::n_cols(P); col++) {
+                const int w = Sp::col_w(P, col);
                 const unsigned char* src = P.col_ptr[col] + (size_t)c.row0 * w;
                 for (int i = c.lane; i < kTile * w; i += 32)
-                    sts_u8(c.stage + P.col_off[col] + i, (i < rows * w) ? src[i] : 0u);
+                    sts_u8(c.stage + Sp::col_off(P, col) + i, (i < rows * w) ? src[i] : 0u);
             }
             __syncwarp();
         } else {
@@ -525,12 +583,13 @@ __device__ __forceinline__ void stage_tile(const KParams& P, const WarpCtx& c, c
 // The tile this warp stages next is pulled into L2 while the current one is processed, so the bulk
 // copy issued at the end of the tile is served from L2 (one stage per warp cannot hide the DRAM
 // latency otherwise).
+template <class Sp>
 __device__ __forceinline__ void prefetch_next(const KParams& P, const Ring& g, uint32_t tile) {
-    if (P.l2_prefetch && elect_one()) {
+    if (Sp::l2_prefetch(P) && elect_one()) {
         const uint64_t nt = (uint64_t)tile + (uint64_t)g.S * g.stride;
         if (nt < g.t_end && (uint32_t)nt != g.guarded_tile)
             for (int c = 0; c < g.n_runs; c++)
-                tma_prefetch_l2(P.run_ptr[c] + (size_t)(uint32_t)nt * P.run_stride[c], P.run_bytes[c]);
+                tma_prefetch_l2(P.run_ptr[c] + (size_t)(uint32_t)nt * Sp::run_stride(P, c), Sp::run_bytes(P, c));
     }
 }
 
@@ -565,13 +624,14 @@ __device__ __forceinline__ int64_t emit_locate(const KParams& P, int lane, unsig
 }
 
 // Materialize (IMPL_EMIT). `valid` is read only.
+template <class Sp>
 __device__ __forceinline__ void sink_emit(const KParams& P, const WarpCtx& c, unsigned valid) {
     int64_t pos = emit_locate(P, c.lane, valid);
     // only the surviving tuples are visited (a selective pass leaves a few per warp tile)
     for (unsigned todo = valid; todo; todo &= todo - 1) {
         const int r = __ffs(todo) - 1;
         if (pos < P.out_cap)
-            for (int k = 0; k < P.n_out; k++) P.out_col[k][pos] = ld_row(P, c, P.out[k], r);
+            for (int k = 0; k < Sp::n_out(P); k++) P.out_col[k][pos] = ld_row(P, c, Sp::out(P, k), r);
         pos++;
     }
 }
@@ -589,14 +649,14 @@ __device__ __forceinline__ void emit_put(const KParams& P, const WarpCtx& c, uns
 
 // End of the scan for IMPL_LOWAGG: warp-reduce the accumulators of the first n groups (at most P.G) and
 // add them to the global group table.
-template <int ND>
+template <class Sp, int ND>
 __device__ __forceinline__ void flush_lowagg(const KParams& P, int lane, int NA, int NK, uint32_t sacc, int n,
                                              const uint64_t (&dk)[ND]) {
-    if (n > P.G) n = P.G;
+    if (n > Sp::G(P)) n = Sp::G(P);
     for (int e = 0; e < n; e++) {
         const int slot = warp_group_slot(P, NK, reg_at(dk, e), lane);
         for (int a = 0; a < NA; a++) {
-            const int kind = P.agg_kind[a];
+            const int kind = Sp::agg_kind(P, a);
             const int64_t v = warp_reduce(lds_b64(sacc + ((e * NA + a) * 32 + lane) * 8), kind);
             if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, v);
         }
@@ -610,9 +670,18 @@ __device__ __forceinline__ void flush_lowagg(const KParams& P, int lane, int NA,
 // ROUNDS (instantiated with GR = 0 and LATE only): sink rounds of a materialize (KParams::n_rounds). Per
 // tile the prefix units run, the output positions are located once, then every round runs its units and
 // stores its values, so the value slots bound one round instead of the whole sink.
+// The spec the kernel reads its host-known fields through: GenericSpec (read from P) in the library, a
+// FixedSpec in a run-time specialization (jit.h), which defines RQ_SCAN_SPEC before including this file.
+// (A macro rather than a template parameter or a wrapper around the body: either would change the
+// ahead-of-time kernels - their names, or their code, since the body would then be compiled as a
+// function of its own before being inlined.)
+#ifndef RQ_SCAN_SPEC
+#define RQ_SCAN_SPEC GenericSpec
+#endif
 template <int GR, bool CROSS = false, bool LATE = false, bool ROUNDS = false>
 __global__ void __launch_bounds__(kMaxWarps * 32, 1)
 rq_scan_kernel(const __grid_constant__ KParams P) {
+    using Sp = RQ_SCAN_SPEC;
     static_assert(!CROSS || GR == 0, "the cross-source variant has the generic sinks only");
     static_assert(!LATE || GR == 0, "the late variant has the generic sinks only");
     static_assert(!ROUNDS || (GR == 0 && !CROSS && LATE), "the round variant is the late one with rounds");
@@ -628,13 +697,13 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     // elect / R2UR loop per copy - 18 instructions per tuple in the first version of this kernel).
     const int warp = __shfl_sync(kFull, (int)(threadIdx.x >> 5), 0);
     const int W = blockDim.x >> 5;
-    const int S = P.stages;
+    const int S = Sp::stages(P);
 
     const uint32_t smem0 = smem_u32(rq_smem);
     const uint32_t bars = smem0 + warp * (kMaxStages * 8);
-    const uint32_t wbase = smem0 + P.warp_off + warp * P.warp_bytes;
+    const uint32_t wbase = smem0 + Sp::warp_off(P) + warp * Sp::warp_bytes(P);
     asm volatile("" : "+r"(lane));
-    const uint32_t sacc = wbase + P.acc_rel;            // GR == 0 low-card path: [g][a][lane] int64
+    const uint32_t sacc = wbase + Sp::acc_rel(P);            // GR == 0 low-card path: [g][a][lane] int64
 
     int64_t n_rows = P.n_rows;
     if (P.n_rows_ptr) { n_rows = *P.n_rows_ptr; if (n_rows > P.n_rows_cap) n_rows = P.n_rows_cap; }
@@ -658,14 +727,14 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     }
     const uint32_t stride = gridDim.x * W;
     const uint32_t first = t_begin + blockIdx.x * W + warp;
-    const int NA = P.na, NK = P.nk;
-    const int sink = P.sink;
+    const int NA = Sp::na(P), NK = Sp::nk(P);
+    const int sink = Sp::sink(P);
 
     // the program, decoded on the host, is copied to shared memory once per CTA
-    const uint32_t prog = smem0 + P.prog_off;
+    const uint32_t prog = smem0 + Sp::prog_off(P);
     {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(P.insn);
-        for (int i = threadIdx.x; i < P.n_insn * 8; i += blockDim.x) sts_b32(prog + i * 4, src[i]);
+        for (int i = threadIdx.x; i < Sp::n_insn(P) * 8; i += blockDim.x) sts_b32(prog + i * 4, src[i]);
     }
     if (!CROSS && lane == 0) {
         for (int s = 0; s < S; s++) mbar_init_s(bars + s * 8, 1);
@@ -687,7 +756,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             rcnt[g] = 0;
 #pragma unroll
             for (int a = 0; a < kNAR; a++) {
-                const uint64_t id = (uint64_t)agg_identity(a < NA ? P.agg_kind[a] : 0);
+                const uint64_t id = (uint64_t)agg_identity(a < NA ? Sp::agg_kind(P, a) : 0);
                 racc[g][2 * a] = (uint32_t)id;
                 racc[g][2 * a + 1] = (uint32_t)(id >> 32);
             }
@@ -707,12 +776,12 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll
             for (int a = 0; a < kNAR; a++) {
                 if (a >= NA) continue;
-                const int kind = P.agg_kind[a];
-                const int mode = P.agg_mode[a];
+                const int kind = Sp::agg_kind(P, a);
+                const int mode = Sp::agg_mode(P, a);
                 uint64_t part;
                 if (kind == RQ_AGG_COUNT) part = rcnt[g];
                 else if (kind == RQ_AGG_SUM && mode == AM_P1) part = racc[g][2 * a];
-                else if (kind == RQ_AGG_SUM && mode == AM_P2) part = (uint64_t)racc[g][2 * a] + ((uint64_t)racc[g][2 * a + 1] << P.agg_shift[a]);
+                else if (kind == RQ_AGG_SUM && mode == AM_P2) part = (uint64_t)racc[g][2 * a] + ((uint64_t)racc[g][2 * a + 1] << Sp::agg_shift(P, a));
                 else part = (uint64_t)racc[g][2 * a] | ((uint64_t)racc[g][2 * a + 1] << 32);
                 const int64_t v = warp_reduce((int64_t)part, kind);
                 if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, v);
@@ -737,13 +806,13 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll
             for (int a = 0; a < kNAR; a++) {
                 if (a >= NA) continue;
-                const int kind = P.agg_kind[a];
-                const int mode = P.agg_mode[a];
+                const int kind = Sp::agg_kind(P, a);
+                const int mode = Sp::agg_mode(P, a);
                 uint64_t part;
                 if (kind == RQ_AGG_COUNT) part = warp_sum_u32(rcnt[g]);
                 else if (kind == RQ_AGG_SUM && mode == AM_P1) { part = warp_sum_u32(racc[g][2 * a]); racc[g][2 * a] = 0; }
                 else if (kind == RQ_AGG_SUM && mode == AM_P2) {
-                    part = warp_sum_u32(racc[g][2 * a]) + (warp_sum_u32(racc[g][2 * a + 1]) << P.agg_shift[a]);
+                    part = warp_sum_u32(racc[g][2 * a]) + (warp_sum_u32(racc[g][2 * a + 1]) << Sp::agg_shift(P, a));
                     racc[g][2 * a] = 0; racc[g][2 * a + 1] = 0;
                 } else continue;
                 if (lane == 0 && slot >= 0) group_table_add(P, slot, a, kind, (int64_t)part);
@@ -753,7 +822,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     };
     int tiles_to_flush = P.flush_tiles;
     if (GR == 0 && sink == IMPL_LOWAGG) {
-        for (int i = lane; i < P.G * NA * 32; i += 32) sts_b64(sacc + i * 8, agg_identity(P.agg_kind[(i >> 5) % NA]));
+        for (int i = lane; i < Sp::G(P) * NA * 32; i += 32) sts_b64(sacc + i * 8, agg_identity(Sp::agg_kind(P, (i >> 5) % NA)));
     }
     __syncwarp();
 
@@ -761,11 +830,11 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
     // scanned data is streamed once, so it is marked evict-first in L2
     const Ring ring{bars, wbase, S, stride, t_end,
                     (P.borrowed && ((uint32_t)n_rows & (kTile - 1)) != 0) ? n_tiles - 1 : 0xffffffffu,
-                    l2_evict_first_policy(), P.n_runs, P.stream_hint != 0};
-    const int n_cols = P.n_cols;
+                    l2_evict_first_policy(), Sp::n_runs(P), Sp::stream_hint(P) != 0};
+    const int n_cols = Sp::n_cols(P);
     if (!CROSS && n_cols > 0) {
         for (int s = 0; s < S; s++)
-            if ((uint64_t)first + (uint64_t)s * stride < t_end) issue_tile(P, ring, first + s * stride, s);
+            if ((uint64_t)first + (uint64_t)s * stride < t_end) issue_tile<Sp>(P, ring, first + s * stride, s);
     }
 
     int s = 0;
@@ -779,13 +848,13 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
             break;
         }
         WarpCtx c;
-        c.stage = wbase + s * P.stage_bytes;
+        c.stage = wbase + s * Sp::stage_bytes(P);
         c.wbase = wbase;
         c.row0 = (int64_t)tile * (int64_t)kTile;
         c.lane = lane;
 
-        stage_tile<CROSS>(P, c, ring, tile, s, phase, n_rows, n_inner, n_cols);
-        if (!CROSS) prefetch_next(P, ring, tile);
+        stage_tile<CROSS, Sp>(P, c, ring, tile, s, phase, n_rows, n_inner, n_cols);
+        if (!CROSS) prefetch_next<Sp>(P, ring, tile);
 
         unsigned valid = 0xffu;
         if (c.row0 + kTile > n_rows) {
@@ -809,15 +878,16 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         int64_t rpos = 0;
         int pc0 = 0;
         for (int rd = -1;; rd++) {     // the parts of the program: units [pc0, n_insn) of part rd
-        const int n_insn = !ROUNDS ? P.n_insn : rd < 0 ? P.prefix_end : (int)P.round_unit_end[rd];
+        const int n_insn = !ROUNDS ? Sp::n_insn(P) : rd < 0 ? P.prefix_end : (int)P.round_unit_end[rd];
+        // (with a fixed spec the loop is unrolled and each unit's switch folds to its one case; a unit
+        // that leaves no tuple ends the part: a jump to program_end there, pc = n_insn here)
+#define RQ_STOP()                                                                             \
+    do {                                                                                      \
+        if constexpr (Sp::kFixed) goto program_end; else pc = n_insn;                         \
+    } while (0)
+#pragma unroll
         for (int pc = pc0; pc < n_insn; pc++) {
-            const uint4 w0 = lds_v4b32(prog + pc * 32), w1 = lds_v4b32(prog + pc * 32 + 16);
-            UInsn in;
-            in.code = (uint8_t)w0.x; in.flags = (uint8_t)(w0.x >> 8); in.gop = (uint8_t)(w0.x >> 16); in.aux = (uint8_t)(w0.x >> 24);
-            in.xkind = (uint8_t)w0.y; in.ykind = (uint8_t)(w0.y >> 8); in.zkind = (uint8_t)(w0.y >> 16);
-            in.xrel = w0.z; in.dstrel = w0.w;
-            in.imm = (int64_t)((uint64_t)w1.x | ((uint64_t)w1.y << 32));
-            in.yrel = w1.z; in.zrel = w1.w;
+            const UInsn in = Sp::insn(P, prog, pc);
             const uint32_t xa = ((in.flags & UF_XSLOT) ? wbase : c.stage) + in.xrel;
             const uint32_t ya = ((in.flags & UF_YSLOT) ? wbase : c.stage) + in.yrel;
             // result handling, expanded inside every case so that t never crosses the switch
@@ -827,7 +897,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         if (in.flags & UF_FILTER) {                                                           \
             _Pragma("unroll") for (int r = 0; r < kR; r++)                                    \
                 if ((t[r] & 0xff) == 0) valid &= ~(1u << r);                                  \
-            if (!__any_sync(kFull, valid != 0)) pc = n_insn;                                  \
+            if (!__any_sync(kFull, valid != 0)) RQ_STOP();                                    \
         }                                                                                     \
     } while (0)
 
@@ -950,7 +1020,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         const unsigned f = (((ok[0] ? 0u : 1u) | (ok[1] ? 0u : 2u)) | ((ok[2] ? 0u : 4u) | (ok[3] ? 0u : 8u))) |       \
                            (((ok[4] ? 0u : 16u) | (ok[5] ? 0u : 32u)) | ((ok[6] ? 0u : 64u) | (ok[7] ? 0u : 128u)));   \
         valid &= ~f;                                                                       \
-        if (!__any_sync(kFull, valid != 0)) pc = n_insn;                                   \
+        if (!__any_sync(kFull, valid != 0)) RQ_STOP();                                     \
     } while (0)
 #define RQ_FCMP(N, OP)                                                                     \
     case U_F##N##_M64: {                                                                   \
@@ -1016,25 +1086,25 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     // resident 32-bit word each, 8 loads in flight); only the survivors walk the
                     // hash table.
                     const DProbe& pr = P.probe[in.aux];
-                    if (pr.fetch) {
+                    if (Sp::pr_fetch(pr, in.aux)) {
                         // second pass of a multi-match expansion: the entry was found (and the tuple
                         // multiplied) by the first pass, only the payload is read here
                         int64_t ei[kR];
-                        fetch_vref(P, c, pr.key[0], ei);
+                        fetch_vref(P, c, Sp::pr_key(pr, in.aux, 0), ei);
 #pragma unroll 1
                         for (int r = 0; r < kR; r++) {
                             if (!((valid >> r) & 1)) continue;
                             const int64_t e = reg_at(ei, r);
-                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)e), e);
+                            put_match<LATE, Sp>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)e), e);
                         }
                         __syncwarp();
                         break;
                     }
-                    if (pr.ht.direct) {
+                    if (Sp::pr_direct(pr, in.aux)) {
                         // direct-address build side: one bit test per tuple (all 8 words of a lane are
                         // fetched together), the payload of a hit is one more load; no walk, no compare
                         int64_t dk8[kR];
-                        fetch_vref(P, c, pr.key[0], dk8);
+                        fetch_vref(P, c, Sp::pr_key(pr, in.aux, 0), dk8);
                         uint32_t w[kR];
 #pragma unroll
                         for (int r = 0; r < kR; r++) {
@@ -1046,20 +1116,20 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             const uint64_t idx = (uint64_t)dk8[r] - (uint64_t)pr.ht.dlo;
                             if (!((w[r] >> (idx & 31)) & 1u)) valid &= ~(1u << r);
                         }
-                        if (!pr.bloom_only) {
+                        if (!Sp::pr_bloom_only(pr, in.aux)) {
                             if constexpr (LATE) {
                                 if (P.late_ref_slot[in.aux] != 0xff) {
-                                    const uint32_t dst = wbase + P.slots_rel + P.late_ref_slot[in.aux] * (kTile * 8);
+                                    const uint32_t dst = wbase + Sp::slots_rel(P) + P.late_ref_slot[in.aux] * (kTile * 8);
 #pragma unroll
                                     for (int r = 0; r < kR; r++)
                                         sts_b64(dst + row_in_tile(r, lane) * 8, (int64_t)((uint64_t)dk8[r] - (uint64_t)pr.ht.dlo));
                                 }
                             }
 #pragma unroll 1
-                            for (int q = 0; q < pr.n_out; q++) {
-                                if (pr.out_slot[q] == 0xff) continue;
-                                const int word = (int)pr.pay_word[q] - 2;      // < 0: the payload repeats the join key
-                                const uint32_t dst = wbase + P.slots_rel + pr.out_slot[q] * (kTile * 8);
+                            for (int q = 0; q < Sp::pr_n_out(pr, in.aux); q++) {
+                                if (Sp::pr_out_slot(pr, in.aux, q) == 0xff) continue;
+                                const int word = Sp::pr_pay_word(pr, in.aux, q) - 2;      // < 0: the payload repeats the join key
+                                const uint32_t dst = wbase + Sp::slots_rel(P) + Sp::pr_out_slot(pr, in.aux, q) * (kTile * 8);
                                 int64_t pv[kR];
 #pragma unroll
                                 for (int r = 0; r < kR; r++) {
@@ -1072,16 +1142,16 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             }
                             __syncwarp();
                         }
-                        if (!__any_sync(kFull, valid != 0)) pc = n_insn;
+                        if (!__any_sync(kFull, valid != 0)) RQ_STOP();
                         break;
                     }
                     const uint64_t cap = pr.ht.cap_mask + 1;
-                    const int pnk = pr.ht.nk;
-                    const bool k1 = pnk == 1 && pr.ht.key_kind[0] == 0;   // one integer key: the usual join
+                    const int pnk = Sp::pr_nk(pr, in.aux);
+                    const bool k1 = pnk == 1 && Sp::pr_key_kind(pr, in.aux, 0) == 0;   // one integer key: the usual join
                     uint64_t h[kR];
                     int64_t kv[kR];
                     if (k1) {
-                        fetch_vref(P, c, pr.key[0], kv);
+                        fetch_vref(P, c, Sp::pr_key(pr, in.aux, 0), kv);
 #pragma unroll
                         for (int r = 0; r < kR; r++) h[r] = hash_int(pr.ht, kv[r]);
                     } else {
@@ -1091,11 +1161,11 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         for (int r = 0; r < kR; r++) {
                             if (!((valid >> r) & 1)) continue;
                             int64_t k[kMaxKeys];
-                            for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, pr.key[j], r);
+                            for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, Sp::pr_key(pr, in.aux, j), r);
                             reg_set(h, r, hash_typed(k, pr.ht.key_kind, pnk));
                         }
                     }
-                    if (pr.ht.bloom != nullptr) {
+                    if (Sp::pr_bloom(pr, in.aux)) {
                         uint32_t w[kR];
 #pragma unroll
                         for (int r = 0; r < kR; r++)
@@ -1106,10 +1176,10 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             if ((w[r] & bits) != bits) valid &= ~(1u << r);
                         }
                     }
-                    if (pr.bloom_only) {
+                    if (Sp::pr_bloom_only(pr, in.aux)) {
                         // semi-join reduction pass of a split pipeline: survivors are materialized
                         // and probed for real by the second pass (engine_exec.inl split_at_probe)
-                        if (!__any_sync(kFull, valid != 0)) pc = n_insn;
+                        if (!__any_sync(kFull, valid != 0)) RQ_STOP();
                         break;
                     }
                     if (k1) {
@@ -1132,14 +1202,14 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                                 if (t == tag && (int64_t)ht_entry(pr.ht, i)[1] == kv[r]) {
                                     if (found < 0) found = (int64_t)i;
                                     matches++;
-                                    if (pr.single) break;
+                                    if (Sp::pr_single(pr, in.aux)) break;
                                 }
                                 i = (i + 1) & pr.ht.cap_mask;
                                 t = *ht_entry(pr.ht, i);
                             }
                             if (found < 0) { valid &= ~(1u << r); continue; }
                             if (matches > 1) atomicAdd(pr.dup_counter, (unsigned long long)(matches - 1));
-                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
+                            put_match<LATE, Sp>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
                         }
                     } else {
                         unsigned todo = valid;
@@ -1148,7 +1218,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                             todo &= todo - 1;
                             const uint64_t hr = reg_at(h, r);
                             int64_t k[kMaxKeys];
-                            for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, pr.key[j], r);
+                            for (int j = 0; j < pnk; j++) k[j] = ld_row(P, c, Sp::pr_key(pr, in.aux, j), r);
                             const uint64_t tag = hr | 2ULL;
                             uint64_t i = hr >> pr.ht.shift;
                             int64_t found = -1;
@@ -1159,23 +1229,25 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                                 if (t == tag && slot_keys_equal(pr.ht, i, k)) {
                                     if (found < 0) found = (int64_t)i;
                                     matches++;
-                                    if (pr.single) break;
+                                    if (Sp::pr_single(pr, in.aux)) break;
                                 }
                                 i = (i + 1) & pr.ht.cap_mask;
                             }
                             if (found < 0) { valid &= ~(1u << r); continue; }
                             if (matches > 1) atomicAdd(pr.dup_counter, (unsigned long long)(matches - 1));
-                            put_match<LATE>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
+                            put_match<LATE, Sp>(P, pr, in.aux, wbase, row_in_tile(r, lane), ht_entry(pr.ht, (uint64_t)found), found);
                         }
                     }
                     __syncwarp();
-                    if (!__any_sync(kFull, valid != 0)) pc = n_insn;
+                    if (!__any_sync(kFull, valid != 0)) RQ_STOP();
                     break;
                 }
                 default: break;
             }
 #undef RQ_FINISH
         }
+    program_end: __attribute__((unused));
+#undef RQ_STOP
         // End of one part of the program. The other variants run the whole program as one part. ROUNDS:
         // the prefix (rd = -1) is followed by the locate and round rd by its stores, then the units of
         // round rd + 1 run. No unit after the prefix drops a tuple, so the positions located once hold
@@ -1214,19 +1286,19 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     // minus one an unused dictionary entry, and neither equals a real key
                     uint64_t key[kR];
                     uint32_t k32[kR];
-                    if (P.key32) {
-                        pack_keys32(P, c, k32);
+                    if (Sp::key32(P)) {
+                        pack_keys32<Sp>(P, c, k32);
 #pragma unroll
                         for (int r = 0; r < kR; r++) {
                             key[r] = k32[r];
                             k32[r] = (valid & (1u << r)) ? k32[r] : 0xffffffffu;
                         }
                     } else {
-                        pack_keys(P, c, key);
+                        pack_keys<Sp>(P, c, key);
                     }
                     for (;;) {
                         uint32_t ct[NG];
-                        if (P.key32) {
+                        if (Sp::key32(P)) {
 #pragma unroll
                             for (int g = 0; g < NG; g++) {
                                 const uint32_t d = g < ngroups ? (uint32_t)dk[g] : 0xfffffffeu;
@@ -1296,12 +1368,12 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     // one descriptor word per aggregate (host: choose_agg_modes): bits 0-2 form
                     // (0 = nothing to do here: COUNT or unused), bit 3 = 64-bit operand in shared
                     // memory at (bit 4 ? warp region : stage) + (desc >> 8)
-                    const uint32_t desc = P.agg_desc[a];
+                    const uint32_t desc = Sp::agg_desc(P, a);
                     const int form = (int)(desc & 7u);
                     if (form == AF_NONE) continue;
                     int64_t v[kR];
                     if (desc & 8u) ld_m64(((desc & 16u) ? c.wbase : c.stage) + (desc >> 8) + lane * 16, v);
-                    else fetch_vref(P, c, P.agg_src[a], v);
+                    else fetch_vref(P, c, Sp::agg_src(P, a), v);
                     const int kind = form == AF_MIN ? RQ_AGG_MIN : RQ_AGG_MAX;
                     if (form == AF_P1) {
 #pragma unroll
@@ -1309,7 +1381,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
 #pragma unroll
                             for (int g = 0; g < NG; g++) racc[g][2 * a] += (uint32_t)v[r] * m[g][r];
                     } else if (form == AF_P2) {
-                        const int sh = P.agg_shift[a];
+                        const int sh = Sp::agg_shift(P, a);
                         const uint32_t lomask = (1u << sh) - 1u;
 #pragma unroll
                         for (int r = 0; r < kR; r++) {
@@ -1358,7 +1430,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     seen |= valid;
                 } else {
                     uint64_t key[kR];
-                    pack_keys(P, c, key);
+                    pack_keys<Sp>(P, c, key);
                     unsigned unk = 0;
 #pragma unroll
                     for (int r = 0; r < kR; r++) {
@@ -1372,7 +1444,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     }
                     while (__any_sync(kFull, unk != 0)) {
                         const uint64_t lk = leader_key(unk, key);
-                        if (ngroups >= P.G) {
+                        if (ngroups >= Sp::G(P)) {
                             if (lane == 0) *P.overflow = 1;
                             unk = 0;
                             break;
@@ -1389,9 +1461,9 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     }
                 }
                 for (int a = 0; a < NA; a++) {
-                    const int kind = P.agg_kind[a];
+                    const int kind = Sp::agg_kind(P, a);
                     int64_t v[kR];
-                    if (kind != RQ_AGG_COUNT) fetch_vref(P, c, P.agg_src[a], v);
+                    if (kind != RQ_AGG_COUNT) fetch_vref(P, c, Sp::agg_src(P, a), v);
                     const uint32_t base = sacc + (a * 32 + lane) * 8;
 #pragma unroll
                     for (int r = 0; r < kR; r++) {
@@ -1409,11 +1481,11 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                 }
             } else if (sink == IMPL_BUILD) {
                 // hash-join build (hashjoin.h:226-256): every tuple claims its own entry.
-                const int bnk = P.ht.nk;
-                if (P.ht.direct) {
+                const int bnk = Sp::ht_nk(P);
+                if (Sp::ht_direct(P)) {
                     // direct-address build: set the key's bit, store its payload words (plain stores)
                     int64_t bk[kR];
-                    fetch_vref(P, c, P.key[0], bk);
+                    fetch_vref(P, c, Sp::key(P, 0), bk);
                     uint32_t was[kR];          // the 8 bit-set atomics of a lane are in flight together
 #pragma unroll
                     for (int r = 0; r < kR; r++) {
@@ -1427,16 +1499,16 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         const uint64_t idx = (uint64_t)bk[r] - (uint64_t)P.ht.dlo;
                         if (idx >= P.ht.dsize) { *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1; continue; }   // outside the proven domain
                         if (was[r] & (1u << (idx & 31))) *const_cast<int32_t*>(P.ht_full + kDupKeyFromHtFull) = 1;     // duplicate key: the host falls back to the hash form
-                        for (int q = 0; q < P.n_out; q++) P.ht.darr[idx * P.ht.dnv + q] = (uint64_t)ld_row(P, c, P.out[q], r);
-                        for (int a = 0; a < NA; a++) P.ht.darr[idx * P.ht.dnv + P.gj_acc_word + a] = (uint64_t)agg_identity(P.agg_kind[a]);
+                        for (int q = 0; q < Sp::n_out(P); q++) P.ht.darr[idx * P.ht.dnv + q] = (uint64_t)ld_row(P, c, Sp::out(P, q), r);
+                        for (int a = 0; a < NA; a++) P.ht.darr[idx * P.ht.dnv + P.gj_acc_word + a] = (uint64_t)agg_identity(Sp::agg_kind(P, a));
                         n_inserted++;
                     }
-                } else if (bnk == 1 && P.ht.key_kind[0] == 0) {
+                } else if (bnk == 1 && Sp::ht_key_kind(P, 0) == 0) {
                     // One integer key. The claims (atomicCAS on the home slot) of a lane's tuples
                     // are issued together: a dense tile costs one atomic round trip per lane; a
                     // tuple whose home slot is taken walks on alone.
                     int64_t bk[kR];
-                    fetch_vref(P, c, P.key[0], bk);
+                    fetch_vref(P, c, Sp::key(P, 0), bk);
                     unsigned long long old[kR];
 #pragma unroll
                     for (int r = 0; r < kR; r++) {
@@ -1457,7 +1529,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         }
                         uint64_t* e = ht_entry(P.ht, slot);
                         e[1] = (uint64_t)bk[r];
-                        for (int q = 0; q < P.n_out; q++) e[2 + q] = (uint64_t)ld_row(P, c, P.out[q], r);
+                        for (int q = 0; q < Sp::n_out(P); q++) e[2 + q] = (uint64_t)ld_row(P, c, Sp::out(P, q), r);
                         if (P.ht.bloom != nullptr) atomicOr(&P.ht.bloom[bloom_word(P.ht, hh)], bloom_bits(P.ht, hh));
                         n_inserted++;
                     }
@@ -1466,23 +1538,23 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     for (int r = 0; r < kR; r++) {
                         if (!((valid >> r) & 1)) continue;
                         int64_t k[kMaxKeys];
-                        for (int j = 0; j < bnk; j++) k[j] = ld_row(P, c, P.key[j], r);
+                        for (int j = 0; j < bnk; j++) k[j] = ld_row(P, c, Sp::key(P, j), r);
                         const uint64_t hh = hash_keys(P.ht, k);
                         uint64_t slot;
                         if (!ht_insert_dup(P.ht, k, hh, &slot, P.ht_full)) { *P.ht_full = 1; continue; }
                         uint64_t* e = ht_entry(P.ht, slot);
-                        for (int q = 0; q < P.n_out; q++) e[1 + bnk + q] = (uint64_t)ld_row(P, c, P.out[q], r);
+                        for (int q = 0; q < Sp::n_out(P); q++) e[1 + bnk + q] = (uint64_t)ld_row(P, c, Sp::out(P, q), r);
                         if (P.ht.bloom != nullptr) atomicOr(&P.ht.bloom[bloom_word(P.ht, hh)], bloom_bits(P.ht, hh));
                         n_inserted++;
                     }
                 }
-            } else if (sink == IMPL_HASHAGG && P.ht.packed) {
+            } else if (sink == IMPL_HASHAGG && Sp::ht_packed(P)) {
                 // GROUP BY whose keys pack into one word (bit fields from the value bounds, < 64 bits):
                 // the entry's first word IS the key (+1, 0 = empty), so claiming a slot and publishing its
                 // key are one atomicCAS - no lock state, no fence, nobody ever waits. The home-slot claims
                 // of a lane's 8 tuples are issued together; aggregates are fire-and-forget atomics.
                 uint64_t key[kR];
-                pack_keys(P, c, key);
+                pack_keys<Sp>(P, c, key);
                 unsigned long long old[kR];
 #pragma unroll
                 for (int r = 0; r < kR; r++) {
@@ -1508,20 +1580,20 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     if (!ok) { *P.ht_full = 1; continue; }
                     if (cur == 0ULL) n_inserted++;
                     uint64_t* acc = ht_entry(P.ht, slot) + 1;
-                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
+                    for (int a = 0; a < NA; a++) atomic_agg<Sp>(P, c, acc, a, r);
                 }
             } else if (sink == IMPL_HASHAGG) {
                 for (unsigned todo = valid; todo; todo &= todo - 1) {
                     const int r = __ffs(todo) - 1;
                     int64_t k[kMaxKeys];
-                    for (int j = 0; j < P.ht.nk; j++) k[j] = ld_row(P, c, P.key[j], r);
+                    for (int j = 0; j < Sp::ht_nk(P); j++) k[j] = ld_row(P, c, Sp::key(P, j), r);
                     const uint64_t hh = hash_keys(P.ht, k);
                     uint64_t slot;
                     bool fresh = false;
                     if (!ht_find_or_insert(P.ht, k, hh, &slot, &fresh, P.ht_full)) { *P.ht_full = 1; continue; }
                     if (fresh) n_inserted++;
-                    uint64_t* acc = ht_entry(P.ht, slot) + 1 + P.ht.nk;
-                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
+                    uint64_t* acc = ht_entry(P.ht, slot) + 1 + Sp::ht_nk(P);
+                    for (int a = 0; a < NA; a++) atomic_agg<Sp>(P, c, acc, a, r);
                 }
             } else if (sink == IMPL_GROUPJOIN) {
                 // GROUP BY on the key of a direct-address join (engine_exec.inl groupjoin_probe): the
@@ -1530,20 +1602,20 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                 // with fire-and-forget atomics; the group's other keys stay in the entry until the
                 // compaction reads them once per group.
                 int64_t gk[kR];
-                fetch_vref(P, c, P.key[0], gk);
+                fetch_vref(P, c, Sp::key(P, 0), gk);
 #pragma unroll 1
                 for (int r = 0; r < kR; r++) {
                     if (!((valid >> r) & 1)) continue;
                     const uint64_t idx = (uint64_t)reg_at(gk, r) - (uint64_t)P.ht.dlo;
                     atomicOr(&P.gj_touched[idx >> 5], 1u << (idx & 31));
                     uint64_t* acc = P.ht.darr + idx * P.ht.dnv + P.gj_acc_word;
-                    for (int a = 0; a < NA; a++) atomic_agg(P, c, acc, a, r);
+                    for (int a = 0; a < NA; a++) atomic_agg<Sp>(P, c, acc, a, r);
                 }
-            } else if (sink == IMPL_EMIT && P.expand_probe >= 0) {
+            } else if (sink == IMPL_EMIT && Sp::expand_probe(P) >= 0) {
                 // multi-match hash join (hashjoin.h:118-165): one output row per key-equal entry.
                 // The probe unit in front only applied the Bloom filter; here every surviving tuple
                 // walks its chain and emits (its values, entry index) once per match.
-                const DProbe& pr = P.probe[P.expand_probe];
+                const DProbe& pr = P.probe[Sp::expand_probe(P)];
                 const uint64_t cap = pr.ht.cap_mask + 1;
                 const int pnk = pr.ht.nk;
 #pragma unroll 1
@@ -1560,8 +1632,8 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                         if (t == tag && slot_keys_equal(pr.ht, i, k)) {
                             const unsigned long long pos = atomicAdd(P.out_count, 1ULL);
                             if ((int64_t)pos < P.out_cap) {
-                                for (int q = 0; q < P.n_out; q++) P.out_col[q][pos] = ld_row(P, c, P.out[q], r);
-                                P.out_col[P.n_out][pos] = (int64_t)i;
+                                for (int q = 0; q < Sp::n_out(P); q++) P.out_col[q][pos] = ld_row(P, c, Sp::out(P, q), r);
+                                P.out_col[Sp::n_out(P)][pos] = (int64_t)i;
                             }
                             if (pr.single) break;
                         }
@@ -1569,7 +1641,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
                     }
                 }
             } else if (sink == IMPL_EMIT) {
-                sink_emit(P, c, valid);
+                sink_emit<Sp>(P, c, valid);
             }
         }
 
@@ -1591,7 +1663,7 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         __syncwarp();
         if (!CROSS && n_cols > 0) {
             const uint64_t nt = (uint64_t)tile + (uint64_t)S * stride;
-            if (nt < t_end) issue_tile(P, ring, (uint32_t)nt, s);
+            if (nt < t_end) issue_tile<Sp>(P, ring, (uint32_t)nt, s);
         }
         if (++s == S) { s = 0; phase ^= 1u; }
         if (GR > 0 && P.flush_tiles > 0 && --tiles_to_flush == 0) {
@@ -1605,10 +1677,11 @@ rq_scan_kernel(const __grid_constant__ KParams P) {
         __syncwarp();
         const int n = flush_groups(NK, ngroups, seen);
         if (GR > 0) flush_regs();
-        else flush_lowagg(P, lane, NA, NK, sacc, n, dk);
+        else flush_lowagg<Sp>(P, lane, NA, NK, sacc, n, dk);
     }
 }
 
+#ifndef __CUDACC_RTC__     // (a run-time compiled specialization, jit.h, needs only the kernel body above)
 // The instantiations of the scan kernel and the one a launch uses: gr is the number of register
 // groups (0, 1 or 4); the cross-source, late and round variants exist for gr = 0 only and take precedence.
 using ScanKernel = void (*)(KParams);
@@ -1902,5 +1975,7 @@ __global__ void rq_transpose_rows(const unsigned char* rows, int64_t n, int tupl
         for (int k = 0; k < width; k++) d[k] = s[k];
     }
 }
+
+#endif  // __CUDACC_RTC__
 
 }  // namespace rq

@@ -129,9 +129,12 @@ def load():
     lib.rq_result_free.argtypes = [C.POINTER(rq_result)]
     lib.rq_dist_unique_id.argtypes = [C.POINTER(C.c_uint8)]
     lib.rq_dist_init.argtypes = [C.c_int, C.c_int, C.POINTER(C.c_uint8)]
-    lib.rq_debug_lower.argtypes = [C.POINTER(rq_plan), C.c_int, C.c_int, C.POINTER(C.c_int32),
-                                   C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
-                                   C.c_int, C.c_char_p, C.c_int64]
+    for f in (lib.rq_debug_lower, lib.rq_debug_specialize):
+        f.argtypes = [C.POINTER(rq_plan), C.c_int, C.c_int, C.POINTER(C.c_int32),
+                      C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                      C.c_int, C.c_char_p, C.c_int64]
+    lib.rq_debug_specialized_launches.restype = C.c_ulonglong
+    lib.rq_debug_specialized_launches.argtypes = [C.c_int]
     _lib = lib
     return lib
 
@@ -139,6 +142,22 @@ def load():
 def debug_lower(plan, pipeline, impl, col_types, col_widths, col_min=None, col_max=None):
     """Host-side lowering of one pipeline to the device program, as text (no GPU needed).
     col_min/col_max: optional per-column value bounds (the upload statistics)."""
+    return _debug_text(load().rq_debug_lower, plan, pipeline, impl, col_types, col_widths, col_min, col_max)
+
+
+def debug_specialize(plan, pipeline, impl, col_types, col_widths, col_min=None, col_max=None):
+    """The run-time specialization of one pipeline's scan kernel (same arguments as debug_lower): the
+    kernel variant, the generated source and the NVRTC / ptxas log, compiled for sm_100a (no GPU needed)."""
+    return _debug_text(load().rq_debug_specialize, plan, pipeline, impl, col_types, col_widths, col_min, col_max)
+
+
+def specialized_launches(captured=False):
+    """Scan launches so far, in this process, that ran a specialized kernel (captured: those of them
+    recorded into the CUDA graph of a replayed plan)."""
+    return int(load().rq_debug_specialized_launches(1 if captured else 0))
+
+
+def _debug_text(fn, plan, pipeline, impl, col_types, col_widths, col_min, col_max):
     lib = load()
 
     class _T:
@@ -154,7 +173,7 @@ def debug_lower(plan, pipeline, impl, col_types, col_widths, col_min=None, col_m
     size = 1 << 16
     while True:       # (long IN lists print one line per set member)
         buf = C.create_string_buffer(size)
-        rc = lib.rq_debug_lower(C.byref(cplan), pipeline, impl, ty, wi, mn, mx, n, buf, len(buf))
+        rc = fn(C.byref(cplan), pipeline, impl, ty, wi, mn, mx, n, buf, len(buf))
         if rc == 0:
             return buf.value.decode()
         msg = lib.rq_last_error().decode()
