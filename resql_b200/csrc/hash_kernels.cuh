@@ -28,7 +28,9 @@ constexpr uint64_t kTagLocked = 1ULL;
 // when somebody raised the table-full flag.
 constexpr uint64_t kFullCheckEvery = 256;
 // A claim that had to walk this far (duplicates, or keys clustering under the order-preserving hash)
-// raises FlagBlock::dup_key; `full` points at FlagBlock::ht_full (rq_internal.h)
+// raises FlagBlock::dup_key; `full` points at FlagBlock::ht_full (rq_internal.h). Only hash-form builds
+// walk, and nothing reads dup_key after them: the host looks at it only behind a direct-address build
+// (run_direct_build), and every build launch starts from cleared flags. The flag is harmless here.
 constexpr uint64_t kLongRun = 1024;
 __device__ __forceinline__ void note_long_run(const int32_t* full) { *const_cast<int32_t*>(full + kDupKeyFromHtFull) = 1; }
 
